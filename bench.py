@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RK3 dynamics step throughput (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--mesh CELLS] [--levels L] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--mesh CELLS] [--levels L] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one atm_srk3 (reference: dynamics/rk_timestep.rg:361-500) over the whole synthetic
 icosahedral mesh.  metric = cell-level updates/s = nCells * nVertLevels * steps / seconds (whole job).
@@ -16,6 +16,10 @@ pinned memory + step + D2H, every step), clocks, gpu_launches.
 --impl reference times the reference's CPU implementation of the path.  The reference is Regent and
 cannot be built here, so this arm runs the oracle port (oracle/, a literal C++ restatement) with all
 host threads on a bounded sample of the same workload.
+
+--dump-outputs DIR writes what the last timed step left in the fields the check scans (CHECK_FIELDS) as DIR/<field>.npy,
+float64: the same seeded sample of rows (entities, every level) at every run with the same --mesh / --levels, so that two
+builds can be compared output for output.
 """
 import argparse
 import json
@@ -39,6 +43,8 @@ E2E_FIELDS = ("u", "ru", "w", "theta_m", "rho_zz", "rw", "rho_p", "rtheta_p", "e
 # the acoustic perturbation variables and the tendencies / diagnostics every task of the step feeds into
 CHECK_FIELDS = ("u", "w", "theta_m", "rho_zz", "ru", "rw", "rho_p", "rtheta_p", "rtheta_pp", "rho_pp", "rw_p", "ru_p", "wwAvg",
                 "ruAvg", "tend_u", "tend_theta", "tend_rho", "pv_edge", "ke", "divergence", "vorticity", "v")
+DUMP_BYTES = 48 << 20    # --dump-outputs: all fields together; a field of the headline mesh is 0.3-0.9 GB, so rows are sampled
+DUMP_SEED = 20260
 
 
 def dt_for(n_cells: int) -> float:
@@ -161,6 +167,20 @@ def merge_checks(parts):
             "finite": finite, "combined_checksum": f"{comb:016x}", "fields": out}
 
 
+def dump_outputs(g, out_dir: str):
+    """CHECK_FIELDS as out_dir/<field>.npy (float64, rows = entities in mesh order, all levels): every row when the fields
+    fit DUMP_BYTES, else the same seeded sample of rows for every field of one entity kind, in ascending order."""
+    from mpas_regent_b200 import _abi
+    os.makedirs(out_dir, exist_ok=True)
+    for n in CHECK_FIELDS:
+        a = g.download_field(n)
+        ent, rows = _abi.FIELD_ENTITY[n], a.shape[0]
+        k = min(rows, max(1, DUMP_BYTES // (len(CHECK_FIELDS) * a[0].nbytes)))
+        if k < rows:
+            a = a[np.sort(np.random.default_rng(DUMP_SEED + ent).permutation(rows)[:k])]
+        np.save(os.path.join(out_dir, n + ".npy"), np.ascontiguousarray(a))
+
+
 def host_threads() -> int:
     """host cores this process may use (torchrun exports OMP_NUM_THREADS=1; the oracle takes an explicit count)."""
     try:
@@ -281,7 +301,11 @@ def main():
     ap.add_argument("--physics", choices=("literal", "corrected"), default="literal",
                     help="literal = the reference as it executes (headline); corrected = acoustic u update + back-substitution + "
                          "recover wired in (SURVEY.md 8f rank 1, MPASB200_PHYSICS_CORRECTED)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the fields the last timed step left (a fixed, seeded sample of rows) to DIR/<field>.npy; one GPU only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -291,6 +315,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs samples the fields of a single partition: run it on one GPU")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: there is no CPU fallback for the product path")
     torch.cuda.set_device(local_rank)
@@ -374,6 +400,8 @@ def main():
         torch.cuda.synchronize(); barrier()
         ms = e0.elapsed_time(e1)
         launches = g.launch_count - launches0
+        if args.dump_outputs:
+            dump_outputs(g, args.dump_outputs)      # the state after the last timed step, before the per-kernel pass advances it
         # ---- the same K steps again with a CUDA-event pair around every launch (on the launching stream): per-kernel times.
         # Kept out of the headline region because two event records per launch inflate a step of ~100 short kernels;
         # graph replay is off here (events cannot bracket the nodes of a replayed graph).
