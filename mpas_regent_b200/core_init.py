@@ -160,9 +160,12 @@ def atm_adv_coef_compression(mesh: Mesh, policy: int, deriv_two: np.ndarray = No
 
 
 def atm_couple_coef_3rd_order(coef: float, adv_coefs_3rd: np.ndarray, zb3_cell: np.ndarray):
-    """dynamics_tasks.rg:303-325: adv_coefs_3rd *= coef on every edge; zb3_cell *= coef at LEVEL 0 only."""
-    adv_coefs_3rd *= coef
-    zb3_cell[:, 0, :] *= coef
+    """dynamics_tasks.rg:303-325: adv_coefs_3rd *= coef on every edge; zb3_cell *= coef at LEVEL 0 only.  Either may be
+    None (the mesh-only half and the 3-D half run apart when the level-0 data is built without any 3-D field)."""
+    if adv_coefs_3rd is not None:
+        adv_coefs_3rd *= coef
+    if zb3_cell is not None:
+        zb3_cell[:, 0, :] *= coef
     return adv_coefs_3rd, zb3_cell
 
 

@@ -61,15 +61,66 @@ def scale_mesh(mesh: Mesh, policy: int, a: float = SPHERE_RADIUS) -> Mesh:
     return Mesh(v=v, partition=mesh.partition, name=mesh.name)
 
 
-def _smooth(rng, x, y, z, nlev1, amp, base=0.0, nmodes=4):
-    """low-order smooth field on the unit sphere x level, amplitude ~amp around base."""
+def _smooth(modes, x, y, z, nlev1, amp, base=0.0):
+    """low-order smooth field on the unit sphere x level, amplitude ~amp around base.  ``modes`` [nmodes, 6] rows
+    (c0, c1, c2, c3, phase, wavenumber) from m5_draws; pointwise in (x, y, z), so any subset of rows evaluates alone."""
     out = np.full((x.shape[0], nlev1), base, dtype=np.float64)
     k = np.arange(nlev1) / max(nlev1 - 1, 1)
-    for _ in range(nmodes):
-        c = rng.normal(size=4)
-        ph = rng.uniform(0, 2 * np.pi)
+    nmodes = len(modes)
+    for c in modes:
         horiz = c[0] * x + c[1] * y + c[2] * z + c[3] * x * y
-        out += amp / nmodes * horiz[:, None] * np.cos(np.pi * rng.integers(1, 3) * k + ph)[None, :]
+        out += amp / nmodes * horiz[:, None] * np.cos(np.pi * c[5] * k + c[4])[None, :]
+    return out
+
+
+def m5_draws(nC: int, nE: int, L: int, seed: int = SEED) -> Dict[str, np.ndarray]:
+    """Every random number the harness draws for the never-written fields (rule M5), in the order make_state has always
+    drawn them: zb3 factor, deriv_two, defc_a / defc_b, ten _smooth mode sets, u_init / v_init, coeffs_reconstruct.
+    Unscaled: make_static scales them with the mesh."""
+    rng = np.random.default_rng(seed)
+    d = dict(zb3_factor=rng.uniform(0.5, 1.5, size=(nE, 1, 2)), deriv_two=rng.normal(size=(nE, 2 * FIFTEEN)),
+             defc_a=rng.normal(size=(nC, MAX_EDGES)), defc_b=rng.normal(size=(nC, MAX_EDGES)))
+    modes = np.zeros((len(M5_SMOOTH), 4, 6))
+    for f in range(len(M5_SMOOTH)):
+        for m in range(4):
+            modes[f, m, :4] = rng.normal(size=4)
+            modes[f, m, 4] = rng.uniform(0, 2 * np.pi)
+            modes[f, m, 5] = rng.integers(1, 3)
+    d["modes"] = modes
+    d["u_init"] = 10.0 + rng.normal(size=L)
+    d["v_init"] = rng.normal(size=L)
+    d["coeffs_reconstruct"] = rng.normal(size=(nC, MAX_EDGES, 3)) * 0.3
+    return d
+
+
+#: the M5 fields built from a _smooth mode set, in draw order: (field, cell or edge, amplitude, base, kind);
+#: kind "factor" multiplies theta_m by (1 + smooth), "one_plus" is 1 + smooth
+M5_SMOOTH = (("h", "cell", 50.0, 1000.0, "plain"), ("rt_diabatic_tend", "cell", 1e-4, 0.0, "plain"),
+             ("t_init", "cell", 0.01, 0.0, "factor"), ("tend_rho_physics", "cell", 1e-6, 0.0, "plain"),
+             ("tend_rtheta_physics", "cell", 1e-3, 0.0, "plain"), ("theta_m_save", "cell", 0.01, 0.0, "factor"),
+             ("tend_ru_physics", "edge", 1e-4, 0.0, "plain"), ("u_tend", "edge", 1e-2, 0.0, "plain"),
+             ("tend_ru", "edge", 1e-2, 0.0, "plain"), ("cqu", "edge", 0.01, 0.0, "one_plus"))
+
+
+def m5_fields(modes: np.ndarray, cell_xyz, edge_xyz, theta_m: np.ndarray, rho_zz: np.ndarray, c1: np.ndarray,
+              c2: np.ndarray) -> Dict[str, np.ndarray]:
+    """The 3-D M5 fields on any set of rows: the _smooth ones are pointwise in the UNIT-sphere coordinates ``cell_xyz`` /
+    ``edge_xyz``; t_init and theta_m_save scale ``theta_m`` of the same cells; rho_edge averages the coupled ``rho_zz`` of
+    the cells c1 / c2 (0-based rows of rho_zz, len(rho_zz) = the zero pad).  Same keys and order as make_state's."""
+    L1 = theta_m.shape[1]
+    lev = np.arange(L1)[None, :] < L1 - 1
+    out = {}
+    rz_p = np.concatenate([rho_zz, np.zeros((1, L1))], 0)
+    for i, (name, ent, amp, base, kind) in enumerate(M5_SMOOTH):
+        if name == "tend_ru_physics":      # rho_edge sits between the cell and the edge fields
+            with np.errstate(invalid="ignore", over="ignore"):
+                out["rho_edge"] = np.where(lev, 0.5 * (rz_p[c1] + rz_p[c2]), 0.0)
+        s = _smooth(modes[i], *(cell_xyz if ent == "cell" else edge_xyz), L1, amp, base)
+        if kind == "factor":
+            s = theta_m * (1.0 + s)
+        elif kind == "one_plus":
+            s = 1.0 + s
+        out[name] = np.where(lev, s, 0.0)
     return out
 
 
@@ -96,21 +147,79 @@ def vertical_grid(L: int, zt: float = 45000.0, strf: float = 1.5):
     return zw, sh, ah, dzw, dzu, vert
 
 
+def make_static(mesh_unit: Mesh, nVertLevels: int, policy: int = CORRECTED, m5: bool = True, seed: int = SEED):
+    """The part of make_state that needs no 3-D array: level-0 ("static") data, the vertical grid with u_init / v_init,
+    and the harness draws (rule M5).  Returns (HostState with static / vert / extras[coeffs_reconstruct, deriv_two] set
+    and no fields, the m5_draws dict or None)."""
+    L = nVertLevels
+    mesh = scale_mesh(mesh_unit, policy)
+    v = mesh.v
+    nC, nE = mesh.nCells, mesh.nEdges
+    st = HostState(nVertLevels=L, policy=policy, mesh=mesh)
+    st.vert = vertical_grid(L)[-1]
+    dr = m5_draws(nC, nE, L, seed) if m5 else None
+    S = st.static
+    S["fVertex"] = 2.0 * OMEGA * np.sin(v["latVertex"])
+    sg = core_init.atm_compute_signs(mesh, policy)
+    deriv_two = dr["deriv_two"] * (0.05 / (v["dcEdge"] ** 2))[:, None] if m5 else None
+    adv = core_init.atm_adv_coef_compression(mesh, policy, deriv_two)
+    adv3, _ = core_init.atm_couple_coef_3rd_order(0.25, adv["adv_coefs_3rd"], None)
+    ms = core_init.atm_compute_mesh_scaling(mesh, policy, True)
+    S.update(nEdgesOnCell=v["nEdgesOnCell"], edgesOnCell=v["edgesOnCell"], verticesOnCell=v["verticesOnCell"],
+             kiteForCell=sg["kiteForCell"], edgesOnCellSign=sg["edgesOnCellSign"], latCell=v["latCell"],
+             cellsOnEdge=v["cellsOnEdge"], verticesOnEdge=v["verticesOnEdge"], nEdgesOnEdge=v["nEdgesOnEdge"],
+             edgesOnEdge_ECP=v["edgesOnEdge"], weightsOnEdge=v["weightsOnEdge"], dcEdge=v["dcEdge"], dvEdge=v["dvEdge"],
+             angleEdge=v["angleEdge"], latEdge=v["latEdge"], nAdvCellsForEdge=adv["nAdvCellsForEdge"],
+             advCellsForEdge=adv["advCellsForEdge"], adv_coefs=adv["adv_coefs"], adv_coefs_3rd=adv3,
+             meshScalingDel2=ms["meshScalingDel2"], meshScalingDel4=ms["meshScalingDel4"],
+             edgesOnVertex=v["edgesOnVertex"], edgesOnVertexSign=sg["edgesOnVertexSign"],
+             kiteAreasOnVertex=v["kiteAreasOnVertex"],
+             xCell=v["xCell"], yCell=v["yCell"], zCell=v["zCell"])
+    S["isShared"] = np.zeros(nC, dtype=np.uint8)
+    S["inCpr"] = np.ones(nC, dtype=np.uint8)
+    S["bdyMaskCell"] = np.zeros(nC, dtype=np.int32)
+    if m5:
+        nEoC = v["nEdgesOnCell"]
+        S["invAreaCell"] = 1.0 / v["areaCell"]
+        S["invDcEdge"] = 1.0 / v["dcEdge"]
+        S["invDvEdge"] = 1.0 / v["dvEdge"]
+        S["invAreaTriangle"] = 1.0 / v["areaTriangle"]
+        S["edgesOnCell_sign"] = sg["edgesOnCellSign"].copy()
+        S["edgesOnVertex_sign"] = sg["edgesOnVertexSign"].copy()
+        S["edgesOnEdge"] = v["edgesOnEdge"].copy()
+        S["specZoneMaskCell"] = np.zeros(nC)
+        S["specZoneMaskEdge"] = np.zeros(nE)
+        slot = (np.arange(MAX_EDGES)[None, :] < nEoC[:, None])
+        S["defc_a"] = np.where(slot, dr["defc_a"], 0.0) / np.sqrt(v["areaCell"])[:, None]
+        S["defc_b"] = np.where(slot, dr["defc_b"], 0.0) / np.sqrt(v["areaCell"])[:, None]
+        st.vert["u_init"][:L] = dr["u_init"]
+        st.vert["v_init"][:L] = dr["v_init"]
+        coeffs = dr["coeffs_reconstruct"]
+    else:
+        coeffs = np.zeros((nC, MAX_EDGES, 3))
+    # inputs of the device-side init chain (mpasb200_init_coupled_diagnostics / mpasb200_reconstruct_2d)
+    S["lonCell"] = v["lonCell"]
+    S["coeffs_reconstruct"] = coeffs
+    st.extras = dict(coeffs_reconstruct=coeffs, deriv_two=deriv_two)
+    return st, dr
+
+
 def make_state(mesh_unit: Mesh, nVertLevels: int, policy: int = CORRECTED, m5: bool = True,
                seed: int = SEED, diag_on_host: bool = True, keep_jw: bool = False) -> HostState:
     """Build every hot-path input.  ``m5`` = fill never-written fields (rule M5); with
-    m5=False they stay zero (rule M1, the literal reading)."""
+    m5=False they stay zero (rule M1, the literal reading).  The level-0 data, the vertical grid and the draws come
+    from make_static; this adds the 3-D fields."""
     L = nVertLevels
     L1 = L + 1
-    mesh = scale_mesh(mesh_unit, policy)
+    st, dr = make_static(mesh_unit, L, policy, m5, seed)
+    mesh = st.mesh
     v = mesh.v
     nC, nE, nV = mesh.nCells, mesh.nEdges, mesh.nVertices
-    rng = np.random.default_rng(seed)
-    st = HostState(nVertLevels=L, policy=policy, mesh=mesh)
     F = st.f
+    S = st.static
 
-    zw, sh, ah, dzw, dzu, vert = vertical_grid(L)
-    st.vert = vert
+    zw, sh, ah, dzw, dzu, _ = vertical_grid(L)
+    vert = st.vert
     u0, t0, t0b, dtdz, eta_t, delta_t = 35.0, 288.0, 250.0, 0.005, 0.2, 4.8e5
     etavs0 = (1.0 - 0.252) * PII / 2.0
     p0 = 1.0e5
@@ -205,7 +314,6 @@ def make_state(mesh_unit: Mesh, nVertLevels: int, policy: int = CORRECTED, m5: b
     F["u"] = u
     rz_p = pad(F["rho_zz"])
     F["ru"] = 0.5 * (rz_p[c1] + rz_p[c2]) * u
-    st.static["fVertex"] = 2.0 * OMEGA * np.sin(v["latVertex"])
 
     # ---- zb (:616-665), zb3 = 0
     z_edge = 0.5 * (zg_p[c1, :] + zg_p[c2, :])
@@ -215,7 +323,7 @@ def make_state(mesh_unit: Mesh, nVertLevels: int, policy: int = CORRECTED, m5: b
     zb[:, :L, 1] = ((z_edge - zg_p[c2]) * (v["dvEdge"] / area_p[c2])[:, None])[:, :L]
     zb3 = np.zeros((nE, L1, 2))
     if m5:   # non-degenerate 3rd-order metric terms
-        zb3[:, :L, :] = 0.1 * zb[:, :L, :] * rng.uniform(0.5, 1.5, size=(nE, 1, 2))
+        zb3[:, :L, :] = 0.1 * zb[:, :L, :] * dr["zb3_factor"]
 
     # ---- rw / w (:681-704): rw accumulates on a zero field
     fzm, fzp = vert["fzm"], vert["fzp"]
@@ -239,11 +347,7 @@ def make_state(mesh_unit: Mesh, nVertLevels: int, policy: int = CORRECTED, m5: b
 
     # ================= atm_core_init chain (atm_core.rg:22-42) =================
     sg = core_init.atm_compute_signs(mesh, policy, zb=zb, zb3=zb3, nlev1=L1)
-    deriv_two = None
-    if m5:
-        deriv_two = rng.normal(size=(nE, 2 * FIFTEEN)) * (0.05 / (v["dcEdge"] ** 2))[:, None]
-    adv = core_init.atm_adv_coef_compression(mesh, policy, deriv_two)
-    adv3, zb3c = core_init.atm_couple_coef_3rd_order(0.25, adv["adv_coefs_3rd"], sg["zb3_cell"])
+    _, zb3c = core_init.atm_couple_coef_3rd_order(0.25, None, sg["zb3_cell"])
     F["zb_cell"], F["zb3_cell"] = sg["zb_cell"], zb3c
 
     # atm_init_coupled_diagnostics (dynamics_tasks.rg:651-725)
@@ -264,7 +368,7 @@ def make_state(mesh_unit: Mesh, nVertLevels: int, policy: int = CORRECTED, m5: b
         e = eoc[:, i]
         fx = np.zeros((nC, L1))
         fx[:, 1:L] = fzm[None, 1:L] * ru_p[e][:, 1:L] + fzp[None, 1:L] * ru_p[e][:, 0:L - 1]
-        term = sg["edgesOnCellSign"][:, i][:, None] * (F["zb_cell"][:, :, i] + np.copysign(1.0, fx) * F["zb3_cell"][:, :, i]) * fx * zf
+        term = S["edgesOnCellSign"][:, i][:, None] * (F["zb_cell"][:, :, i] + np.copysign(1.0, fx) * F["zb3_cell"][:, :, i]) * fx * zf
         rwn[:, 1:L] -= np.where(use, term, 0.0)[:, 1:L]
     F["rw"] = rwn
     rho_base = F["rho_base"]
@@ -281,70 +385,21 @@ def make_state(mesh_unit: Mesh, nVertLevels: int, policy: int = CORRECTED, m5: b
     F["exner_base"] = np.where(lev, exb, 0.0)
     F["pressure_p"] = np.where(lev, zz * RGAS * (F["exner"] * F["rtheta_p"] + rtb * (F["exner"] - F["exner_base"])), 0.0)
 
-    ms = core_init.atm_compute_mesh_scaling(mesh, policy, True)
     F["dss"] = core_init.atm_compute_damping_coefs(zgrid, v["meshDensity"], L)
 
-    # ---- level-0 ("static") data -------------------------------------------------
-    S = st.static
-    S.update(nEdgesOnCell=v["nEdgesOnCell"], edgesOnCell=v["edgesOnCell"], verticesOnCell=v["verticesOnCell"],
-             kiteForCell=sg["kiteForCell"], edgesOnCellSign=sg["edgesOnCellSign"], latCell=v["latCell"],
-             cellsOnEdge=v["cellsOnEdge"], verticesOnEdge=v["verticesOnEdge"], nEdgesOnEdge=v["nEdgesOnEdge"],
-             edgesOnEdge_ECP=v["edgesOnEdge"], weightsOnEdge=v["weightsOnEdge"], dcEdge=v["dcEdge"], dvEdge=v["dvEdge"],
-             angleEdge=v["angleEdge"], latEdge=v["latEdge"], nAdvCellsForEdge=adv["nAdvCellsForEdge"],
-             advCellsForEdge=adv["advCellsForEdge"], adv_coefs=adv["adv_coefs"], adv_coefs_3rd=adv3,
-             meshScalingDel2=ms["meshScalingDel2"], meshScalingDel4=ms["meshScalingDel4"],
-             edgesOnVertex=v["edgesOnVertex"], edgesOnVertexSign=sg["edgesOnVertexSign"],
-             kiteAreasOnVertex=v["kiteAreasOnVertex"],
-             xCell=v["xCell"], yCell=v["yCell"], zCell=v["zCell"])
-    S["isShared"] = np.zeros(nC, dtype=np.uint8)
-    S["inCpr"] = np.ones(nC, dtype=np.uint8)
-    S["bdyMaskCell"] = np.zeros(nC, dtype=np.int32)
-
     # ---- fields the reference never writes (M1: zero;  M5: deterministic non-degenerate values)
-    xc, yc, zc = (mesh_unit.v[k] for k in ("xCell", "yCell", "zCell"))
-    xe, ye, ze = (mesh_unit.v[k] for k in ("xEdge", "yEdge", "zEdge"))
-    zero_c = lambda: np.zeros((nC, L1))
-    zero_e = lambda: np.zeros((nE, L1))
     if m5:
-        S["invAreaCell"] = 1.0 / v["areaCell"]
-        S["invDcEdge"] = 1.0 / v["dcEdge"]
-        S["invDvEdge"] = 1.0 / v["dvEdge"]
-        S["invAreaTriangle"] = 1.0 / v["areaTriangle"]
-        S["edgesOnCell_sign"] = sg["edgesOnCellSign"].copy()
-        S["edgesOnVertex_sign"] = sg["edgesOnVertexSign"].copy()
-        S["edgesOnEdge"] = v["edgesOnEdge"].copy()
-        S["specZoneMaskCell"] = np.zeros(nC)
-        S["specZoneMaskEdge"] = np.zeros(nE)
-        slot = (np.arange(MAX_EDGES)[None, :] < nEoC[:, None])
-        S["defc_a"] = np.where(slot, rng.normal(size=(nC, MAX_EDGES)), 0.0) / np.sqrt(v["areaCell"])[:, None]
-        S["defc_b"] = np.where(slot, rng.normal(size=(nC, MAX_EDGES)), 0.0) / np.sqrt(v["areaCell"])[:, None]
-        lev_c = (np.arange(L1)[None, :] < L)
-        F["h"] = np.where(lev_c, _smooth(rng, xc, yc, zc, L1, 50.0, 1000.0), 0.0)
-        F["rt_diabatic_tend"] = np.where(lev_c, _smooth(rng, xc, yc, zc, L1, 1e-4), 0.0)
-        F["t_init"] = np.where(lev_c, F["theta_m"] * (1.0 + _smooth(rng, xc, yc, zc, L1, 0.01)), 0.0)
-        F["tend_rho_physics"] = np.where(lev_c, _smooth(rng, xc, yc, zc, L1, 1e-6), 0.0)
-        F["tend_rtheta_physics"] = np.where(lev_c, _smooth(rng, xc, yc, zc, L1, 1e-3), 0.0)
-        F["theta_m_save"] = np.where(lev_c, F["theta_m"] * (1.0 + _smooth(rng, xc, yc, zc, L1, 0.01)), 0.0)
-        F["rho_edge"] = np.where(lev_c, 0.5 * (rz_p[c1] + rz_p[c2]), 0.0)
-        F["tend_ru_physics"] = np.where(lev_c, _smooth(rng, xe, ye, ze, L1, 1e-4), 0.0)
-        F["u_tend"] = np.where(lev_c, _smooth(rng, xe, ye, ze, L1, 1e-2), 0.0)
-        F["tend_ru"] = np.where(lev_c, _smooth(rng, xe, ye, ze, L1, 1e-2), 0.0)
-        F["cqu"] = np.where(lev_c, 1.0 + _smooth(rng, xe, ye, ze, L1, 0.01), 0.0)
-        vert["u_init"][:L] = 10.0 + rng.normal(size=L)
-        vert["v_init"][:L] = rng.normal(size=L)
-        coeffs = rng.normal(size=(nC, MAX_EDGES, 3)) * 0.3
+        F.update(m5_fields(dr["modes"], [mesh_unit.v[k] for k in ("xCell", "yCell", "zCell")],
+                           [mesh_unit.v[k] for k in ("xEdge", "yEdge", "zEdge")], F["theta_m"], F["rho_zz"], c1, c2))
     else:
         for k in ("h", "rt_diabatic_tend", "t_init", "tend_rho_physics", "tend_rtheta_physics", "theta_m_save"):
-            F[k] = zero_c()
+            F[k] = np.zeros((nC, L1))
         for k in ("rho_edge", "tend_ru_physics", "u_tend", "tend_ru", "cqu"):
-            F[k] = zero_e()
-        coeffs = np.zeros((nC, MAX_EDGES, 3))
+            F[k] = np.zeros((nE, L1))
+    coeffs, deriv_two = st.extras["coeffs_reconstruct"], st.extras["deriv_two"]
     st.extras = dict(coeffs_reconstruct=coeffs, theta_base=theta_base, zb=zb, zb3=zb3, deriv_two=deriv_two)
     if keep_jw:
         st.extras["jw"] = jw_snapshot
-    # inputs of the device-side init chain (mpasb200_init_coupled_diagnostics / mpasb200_reconstruct_2d)
-    S["lonCell"] = v["lonCell"]
-    S["coeffs_reconstruct"] = coeffs
     F["theta_base"] = theta_base
     F["uReconstructZonal"], F["uReconstructMeridional"] = core_init.mpas_reconstruct_2d(mesh, policy, F["u"], coeffs, L)
     # v is produced by atm_compute_solve_diagnostics(rk_step=-1) at init (atm_core.rg:31): that is a
@@ -361,3 +416,47 @@ def make_state(mesh_unit: Mesh, nVertLevels: int, policy: int = CORRECTED, m5: b
     for k in list(F):
         F[k] = np.ascontiguousarray(F[k], dtype=np.float64)
     return st
+
+
+# ---- the same state built on the device, one handle per partition -----------------------------------------------------
+def jw_inputs(mesh_unit: Mesh, st: HostState, draws: Dict[str, np.ndarray], lm=None) -> Dict[str, np.ndarray]:
+    """Per-entity inputs of init_on_device for the rows one handle holds (``lm`` a partition.LocalMesh, None = the whole
+    mesh): latCell / areaCell / meshDensity / latVertex of the scaled mesh, the unit-sphere coordinates of cells and edges
+    (rows x, y, z), the zb3 factors of the edges, and the _smooth mode sets (global)."""
+    v, u = st.mesh.v, mesh_unit.v
+    c, e, vx = (slice(None), slice(None), slice(None)) if lm is None else (lm.cells, lm.edges, lm.vertices)
+    return dict(latCell=v["latCell"][c], areaCell=v["areaCell"][c], meshDensity=v["meshDensity"][c], latVertex=v["latVertex"][vx],
+                cell_xyz=np.stack([u[k][c] for k in ("xCell", "yCell", "zCell")]),
+                edge_xyz=np.stack([u[k][e] for k in ("xEdge", "yEdge", "zEdge")]),
+                zb3_factor=np.ascontiguousarray(draws["zb3_factor"][e]), modes=draws["modes"])
+
+
+def init_on_device(dyn, static: Dict[str, np.ndarray], jw: Dict[str, np.ndarray], vert: Dict[str, np.ndarray]) -> None:
+    """make_state(m5=True)'s 3-D fields built on a handle whose mesh (``static``, from make_static or a static shard) is
+    uploaded: init_atm_case_jw, rho_zz *= zz, zb3, zb_cell, the level-0 zb3 coupling, atm_init_coupled_diagnostics,
+    atm_compute_damping_coefs, mpas_reconstruct_2d, then the M5 fields of the rows held (from the device theta_m and
+    coupled rho_zz).  CORRECTED index policy.
+
+    On a local mesh every owned entity comes out right; ghost ring 2 and the edges to cells that are not held do not
+    (their stencils leave the rows held) until parallel.INIT_EXCHANGE runs.  atm_compute_solve_diagnostics(-1) is the
+    caller's, as with uploaded inputs."""
+    assert dyn.cfg.index_policy == CORRECTED, "init_on_device builds the CORRECTED reading"
+    L = dyn.dims.nVertLevels
+    dyn.init_atm_case_jw(jw["latCell"], jw["areaCell"], jw["latVertex"])
+    with np.errstate(all="ignore"):          # rows outside the stencil's reach may hold inf / NaN until the exchange
+        dyn.upload_field("rho_zz", dyn.download_field("rho_zz") * dyn.download_field("zz"))   # atm_init_coupled_diagnostics divides by zz
+        zb = dyn.download_field("zb")
+        zb3 = np.zeros_like(zb)
+        zb3[:, :L, :] = 0.1 * zb[:, :L, :] * jw["zb3_factor"]
+    dyn.upload_field("zb3", zb3)
+    dyn.atm_compute_zb_cell()
+    dyn.atm_couple_coef_3rd_order(0.25)
+    dyn.atm_init_coupled_diagnostics()
+    dyn.atm_compute_damping_coefs(jw["meshDensity"])
+    dyn.mpas_reconstruct_2d(False, True)
+    nC = dyn.dims.nCells
+    c1, c2 = (resolve_ids(static["cellsOnEdge"][:, i], nC, CORRECTED) for i in (0, 1))
+    with np.errstate(all="ignore"):
+        F = m5_fields(jw["modes"], list(jw["cell_xyz"]), list(jw["edge_xyz"]), dyn.download_field("theta_m"),
+                      dyn.download_field("rho_zz"), c1, c2)
+    dyn.upload_state(F, {k: vert[k] for k in ("u_init", "v_init", "cofrz")})

@@ -58,6 +58,33 @@ EXCHANGES_CORRECTED: Dict[str, Dict[str, List[str]]] = {
 }
 
 
+#: init_jw.init_on_device run on a local mesh computes every owned entity right (its stencils reach ring 1 at most) but
+#: leaves ghost ring 2 and the edges to cells not held wrong (inf / NaN on some); this one exchange after it copies every
+#: cell and edge field the device init writes from owner to holder, after which each rank equals the single-partition
+#: device init restricted to its rows, ghosts included.
+INIT_EXCHANGE: Dict[str, List[str]] = {
+    "cell": ["zgrid", "zz", "rho_base", "pressure_p", "rho_p", "theta_base", "exner", "theta_m", "rtheta_p", "rho_zz", "rw", "w",
+             "zb_cell", "zb3_cell", "rtheta_base", "exner_base", "pressure_base", "dss", "uReconstructX", "uReconstructY",
+             "uReconstructZ", "uReconstructZonal", "uReconstructMeridional", "h", "rt_diabatic_tend", "t_init", "tend_rho_physics",
+             "tend_rtheta_physics", "theta_m_save"],
+    "edge": ["zxu", "u", "ru", "zb", "zb3", "rho_edge", "tend_ru_physics", "u_tend", "tend_ru", "cqu"],
+}
+
+#: k_pack / k_unpack move at most this many buffer entries (fields x slots) per launch (mpasb200_pack)
+PACK_MAX_ENTRIES = 32
+
+
+def pack_groups(names: Sequence[str]) -> List[List[str]]:
+    """split a field list into consecutive groups that one pack / unpack launch can carry"""
+    groups, n = [[]], 0
+    for name in names:
+        s = FIELD_SLOTS[name]
+        if n + s > PACK_MAX_ENTRIES:
+            groups.append([]); n = 0
+        groups[-1].append(name); n += s
+    return groups
+
+
 def exchange_key(name: str, args=()) -> str:
     """hook key of a task call: the first acoustic step of a stage (small_step == 0) has its own."""
     return "advance_acoustic_step:first" if name == "advance_acoustic_step" and len(args) >= 2 and int(args[1]) == 0 else name
@@ -194,16 +221,17 @@ class NcclExchanger(Exchanger):
             return self.plans[key]
         torch, dist = self.torch, self.dist
         items, ops = [], []
-        for ent, names in spec.items():
-            E, nf = self.ent[ent], sum(FIELD_SLOTS[n] for n in names)       # one buffer entry per slot of an array-typed field
-            row = nf * self.L1
-            sbuf = torch.empty(max(E["ns"] * row, 1), dtype=torch.float64, device="cuda")
-            rbuf = torch.empty(max(E["nr"] * row, 1), dtype=torch.float64, device="cuda")
-            for i, p in enumerate(E["peers_s"]):
-                ops.append(dist.P2POp(dist.isend, sbuf[E["s_off"][i] * row:E["s_off"][i + 1] * row], p))
-            for i, p in enumerate(E["peers_r"]):
-                ops.append(dist.P2POp(dist.irecv, rbuf[E["r_off"][i] * row:E["r_off"][i + 1] * row], p))
-            items.append((E, list(names), sbuf, rbuf))
+        for ent, all_names in spec.items():
+            for names in pack_groups(all_names):
+                E, nf = self.ent[ent], sum(FIELD_SLOTS[n] for n in names)       # one buffer entry per slot of an array-typed field
+                row = nf * self.L1
+                sbuf = torch.empty(max(E["ns"] * row, 1), dtype=torch.float64, device="cuda")
+                rbuf = torch.empty(max(E["nr"] * row, 1), dtype=torch.float64, device="cuda")
+                for i, p in enumerate(E["peers_s"]):
+                    ops.append(dist.P2POp(dist.isend, sbuf[E["s_off"][i] * row:E["s_off"][i + 1] * row], p))
+                for i, p in enumerate(E["peers_r"]):
+                    ops.append(dist.P2POp(dist.irecv, rbuf[E["r_off"][i] * row:E["r_off"][i + 1] * row], p))
+                items.append((E, names, sbuf, rbuf))
         self.plans[key] = (items, ops)
         return self.plans[key]
 
@@ -379,8 +407,9 @@ class DistributedDynamics:
 
 
 # ---- shards --------------------------------------------------------------------------------------------------
-def make_shards(st, world: int, colours: Optional[np.ndarray] = None):
-    """partition a global HostState (CORRECTED policy) into per-rank {lm, static, f, vert}."""
+def make_static_shards(st, world: int, colours: Optional[np.ndarray] = None):
+    """partition the level-0 data of a HostState (CORRECTED policy; init_jw.make_static is enough, no 3-D field is read)
+    into per-rank {lm, static}, launch classes included."""
     mesh = st.mesh
     n_global = (mesh.nCells, mesh.nEdges, mesh.nVertices)
     col = colours if colours is not None else (mesh.partition if mesh.partition is not None and mesh.partition.max() + 1 == world
@@ -393,7 +422,17 @@ def make_shards(st, world: int, colours: Optional[np.ndarray] = None):
     partition.build_halo_lists(locs)
     for lm, loc in zip(locs, statics):
         loc["cellClass"], loc["edgeClass"] = launch_classes(lm, loc)
-    return [dict(lm=lm, static=loc, f=split_state(st.f, lm), vert=dict(st.vert)) for lm, loc in zip(locs, statics)]
+    return [dict(lm=lm, static=loc) for lm, loc in zip(locs, statics)]
+
+
+def make_shards(st, world: int, colours: Optional[np.ndarray] = None):
+    """partition a global HostState (CORRECTED policy) into per-rank {lm, static, f, vert}."""
+    return [dict(lm=sh["lm"], static=sh["static"], f=split_state(st.f, sh["lm"]), vert=dict(st.vert))
+            for sh in make_static_shards(st, world, colours)]
+
+
+#: the array dictionaries a shard may carry: level-0 data, 3-D fields, vertical fields, inputs of init_jw.init_on_device
+SHARD_PARTS = ("static", "f", "vert", "jw")
 
 
 def save_shard(path: str, sh):
@@ -408,7 +447,9 @@ def save_shard(path: str, sh):
         for peer, idx in lm.recv[ent].items():
             meta[f"recv_{ent}_{peer}"] = idx
     np.savez(os.path.join(path, "lm.npz"), **meta)
-    for sub in ("static", "f", "vert"):
+    for sub in SHARD_PARTS:
+        if sub not in sh:
+            continue
         os.makedirs(os.path.join(path, sub), exist_ok=True)
         for k, a in sh[sub].items():
             np.save(os.path.join(path, sub, k + ".npy"), a)
@@ -427,7 +468,9 @@ def load_shard(path: str):
                 _, ent, peer = k.split("_")
                 getattr(lm, kind)[ent][int(peer)] = z[k]
     out = dict(lm=lm)
-    for sub in ("static", "f", "vert"):
+    for sub in SHARD_PARTS:
         d = os.path.join(path, sub)
+        if not os.path.isdir(d):
+            continue
         out[sub] = {f[:-4]: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d)) if f.endswith(".npy")}
     return out
