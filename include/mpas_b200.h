@@ -348,6 +348,41 @@ typedef struct {
 int  mpasb200_set_global_ids(mpasb200_t *h, int entity, const int32_t *global_id, int32_t n);   /* null: back to identity */
 int  mpasb200_summarize_field(mpasb200_t *h, int field, int32_t n_first, int32_t nlevels, MpasFieldSummary *out);
 
+/* ---- exact global integrals (summarize_timestep's scan extended by a sum) ------------------------------------------ *
+ * I = the EXACT sum over entities i < n_first of the caller's numbering and levels k < nlevels of
+ *       p(i,k) = ((a[i,k] * b[i,k]) * wh[i]) * wv[k]
+ * where every product is one IEEE multiply rounded to nearest, in exactly that order; b (field_b = -1), wh (weight_id = -1)
+ * and wv (null) default to 1.  NaN, +Inf and -Inf products are counted and left out of the sum.  The finite products are
+ * added into a fixed-point accumulator without rounding, so the result does not depend on the block schedule, the
+ * renumbering or the partition: the integrals of the owned entities of N ranks, merged with mpasb200_integral_merge, have
+ * the same bits at every N, and a Legion caller may use the merge as a reduction operator over partitions.
+ *
+ * Representation of MpasIntegral: the sum is   sum_{j=0}^{67} limb[j] * 2^(32*j - 1088)   exactly, as integers.  That
+ * covers 2^-1088 .. 2^1088, enough for any sum of up to 2^40 doubles, subnormals included (a double is a multiple of
+ * 2^-1074 below 2^1024).  Any int64 limbs form a valid accumulator.  Every result of the library is in canonical form:
+ * limbs 0..66 in [0, 2^32) and limb 67 signed, so two equal sums have equal limbs.  count = the products taken
+ * (n_first * nlevels, non-finite ones included); n_nan, n_pinf, n_ninf = the products left out.
+ *
+ * register_weights uploads wh once: w[n] in the caller's numbering, n = the entity count of the handle.
+ * integrate is synchronous (host-visible point) and refused during graph capture.  wv is a host array [nlevels].  It
+ * returns MPASB200_EINVAL for an unknown field, slot or weight id, a vertical field, field_b or the weights on another
+ * entity type than field_a, and n_first outside [0, count] or nlevels outside [1, nVertLevels+1].
+ * integral_merge and integral_value need no handle and no GPU.  merge: acc += x, exact, associative and commutative
+ * (MPASB200_EINVAL only if the sum leaves the range above).  value: the sum rounded once, to nearest with ties to even;
+ * +-Inf on overflow, +0.0 for an exact zero.  Any NaN, or both signs of infinity, gives NaN; one sign of infinity alone
+ * gives that infinity.                                                                                                  */
+#define MPASB200_INTEGRAL_LIMBS 68
+#define MPASB200_INTEGRAL_BIAS  1088
+typedef struct {
+  int64_t limb[MPASB200_INTEGRAL_LIMBS];
+  int64_t count, n_nan, n_pinf, n_ninf;
+} MpasIntegral;
+int  mpasb200_register_weights(mpasb200_t *h, int entity, const double *w, int32_t n, int32_t *weight_id);
+int  mpasb200_integrate(mpasb200_t *h, int field_a, int slot_a, int field_b, int slot_b, int weight_id, const double *wv,
+                        int32_t n_first, int32_t nlevels, MpasIntegral *out);
+int  mpasb200_integral_merge(MpasIntegral *acc, const MpasIntegral *x);
+double mpasb200_integral_value(const MpasIntegral *x);
+
 /* ---- halo exchange building blocks (one process per GPU; the wire is the host's job) ------ *
  * Lists are LOCAL entity indices in the caller's (un-renumbered) numbering.  pack gathers
  * `n` columns x `nfields` fields x (nVertLevels+1) levels into the contiguous device

@@ -111,6 +111,15 @@ class MpasFieldSummary(C.Structure):
                 "count": int(self.count), "checksum": f"{int(self.checksum):016x}"}
 
 
+INTEGRAL_LIMBS, INTEGRAL_BIAS = 68, 1088     # MpasIntegral: sum = sum_j limb[j] * 2^(32 j - INTEGRAL_BIAS), exactly
+
+
+class MpasIntegral(C.Structure):
+    """image of MpasIntegral (mpas_b200.h): an exact global integral as a fixed-point accumulator, plus its counts"""
+    _fields_ = [("limb", C.c_int64 * INTEGRAL_LIMBS), ("count", C.c_int64), ("n_nan", C.c_int64), ("n_pinf", C.c_int64),
+                ("n_ninf", C.c_int64)]
+
+
 INIT_MESH_MEMBERS = (
     ("nEdgesOnCell", np.int32, CELL, 1), ("edgesOnCell", np.int32, CELL, "maxEdges"), ("verticesOnCell", np.int32, CELL, "maxEdges"),
     ("cellsOnCell", np.int32, CELL, "maxEdges"), ("cellsOnEdge", np.int32, EDGE, 2), ("verticesOnEdge", np.int32, EDGE, 2),

@@ -2151,3 +2151,110 @@ __global__ void k_summarize_loc(const double* __restrict__ field, const int* __r
     if (key == kmax) atomicMin(&acc->loc_max, id);
   }
 }
+
+// ============================================================================================
+// Exact global integrals (an extension of summarize_timestep): the exact sum over entities i < n (caller's numbering) and
+// levels k < nlev of p = ((a * b) * wh[i]) * wv[k], every product one multiply rounded to nearest in that order (b, wh, wv
+// absent = 1).  NaN / +Inf / -Inf products are counted and left out; every finite product enters a fixed-point
+// superaccumulator whose limb j holds a signed multiple of 2^(32 j - IACC_BIAS).  A double is m * 2^e with m < 2^53 and
+// e >= -1074, so it lands as three 32-bit digits in limbs j, j+1, j+2 with j = (e + IACC_BIAS) / 32 <= 64.  Integer addition
+// is associative, so nothing here depends on the grid, the block schedule, the renumbering or the partition.
+// Each warp owns one accumulator in shared memory.  When every product of one warp-wide iteration falls in the same two
+// limb positions (the usual case: a field spans few binades), the warp sums the digits over its lanes and one lane adds
+// four limbs; otherwise each lane adds its own three digits.  Either way one iteration moves a limb by less than
+// 32 * 2^32 = 2^37, and the warp folds the carries of its accumulator (limbs 0..66 back into [0, 2^32)) every
+// IACC_FOLD_EVERY iterations, so no int64 limb can overflow however many products one warp takes.
+constexpr int IACC_LIMBS = 68;          // MPASB200_INTEGRAL_LIMBS
+constexpr int IACC_BIAS = 1088;         // limb 0 weighs 2^-1088
+constexpr int IACC_FOLD_EVERY = 1 << 24;
+constexpr int IACC_WARPS = 8;           // blockDim.x = 32 * IACC_WARPS
+struct IntAcc { long long limb[IACC_LIMBS]; unsigned long long n_nan, n_pinf, n_ninf; };
+
+DI void iacc_fold(long long* a) {       // limbs 0..66 into [0, 2^32), the carries into limb 67 (arithmetic shifts)
+  long long c = 0;
+  for (int j = 0; j < IACC_LIMBS - 1; ++j) { const long long v = a[j] + c; a[j] = v & 0xffffffffLL; c = v >> 32; }
+  a[IACC_LIMBS - 1] += c;
+}
+DI long long warp_sum_ll(long long v) {
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+DI void iacc_add(long long* a, int j, long long v) {
+  if (v) atomicAdd(reinterpret_cast<unsigned long long*>(a + j), (unsigned long long)v);   // two's complement: a signed add
+}
+
+__global__ void __launch_bounds__(32 * IACC_WARPS)
+k_integrate(const double* __restrict__ fa, const double* __restrict__ fb, const int* __restrict__ map,
+            const double* __restrict__ wh, const double* __restrict__ wv, int n, int nlev, int LP, IntAcc* __restrict__ out) {
+  __shared__ long long acc[IACC_WARPS][IACC_LIMBS];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int j = lane; j < IACC_LIMBS; j += 32) acc[w][j] = 0;
+  __syncwarp();
+  unsigned long long nn = 0, np = 0, nm = 0;
+  const size_t total = (size_t)n * nlev;
+  int iters = 0;
+  // the loop runs warp-uniformly (lanes past the end take part with no product) so that the full-mask collectives are legal
+  for (size_t base = ((size_t)blockIdx.x * IACC_WARPS + w) * 32; base < total; base += (size_t)gridDim.x * blockDim.x) {
+    const size_t t = base + lane;
+    bool fin = false;
+    int j = 0;
+    long long d0 = 0, d1 = 0, d2 = 0;
+    if (t < total) {
+      const int i = (int)(t / nlev), k = (int)(t % nlev);
+      const size_t at = (size_t)map[i] * LP + k;
+      double p = fa[at];
+      if (fb) p = __dmul_rn(p, fb[at]);
+      if (wh) p = __dmul_rn(p, wh[i]);
+      if (wv) p = __dmul_rn(p, wv[k]);
+      if (p != p) nn++;
+      else if (isinf(p)) { if (p > 0) np++; else nm++; }
+      else if (p != 0.0) {
+        const unsigned long long bits = (unsigned long long)__double_as_longlong(p);
+        const int ex = (int)((bits >> 52) & 0x7ff);
+        unsigned long long m = bits & 0xfffffffffffffULL;
+        if (ex) m |= 1ULL << 52;
+        const int s = (ex ? ex - 1075 : -1074) + IACC_BIAS;     // bit position of m's unit, >= 14
+        const int r = s & 31;
+        j = s >> 5;
+        const unsigned long long lo = m << r, hi = r ? m >> (64 - r) : 0ULL;   // m * 2^r < 2^85
+        d0 = (long long)(lo & 0xffffffffULL); d1 = (long long)(lo >> 32); d2 = (long long)hi;
+        if (bits >> 63) { d0 = -d0; d1 = -d1; d2 = -d2; }
+        fin = true;
+      }
+    }
+    const unsigned jmin = __reduce_min_sync(0xffffffffu, fin ? (unsigned)j : 0xffffffffu);
+    if (jmin != 0xffffffffu) {
+      const unsigned jmax = __reduce_max_sync(0xffffffffu, fin ? (unsigned)j : 0u);
+      if (jmax - jmin <= 1) {             // jmin + 3 <= 67
+        const bool up = fin && (unsigned)j != jmin;
+        long long w0 = up ? 0 : d0, w1 = up ? d0 : d1, w2 = up ? d1 : d2, w3 = up ? d2 : 0;
+        w0 = warp_sum_ll(w0); w1 = warp_sum_ll(w1); w2 = warp_sum_ll(w2); w3 = warp_sum_ll(w3);
+        if (lane == 0) { iacc_add(acc[w], jmin, w0); iacc_add(acc[w], jmin + 1, w1); iacc_add(acc[w], jmin + 2, w2); iacc_add(acc[w], jmin + 3, w3); }
+      } else if (fin) {
+        iacc_add(acc[w], j, d0); iacc_add(acc[w], j + 1, d1); iacc_add(acc[w], j + 2, d2);
+      }
+    }
+    if (++iters == IACC_FOLD_EVERY) {
+      __syncwarp();
+      if (lane == 0) iacc_fold(acc[w]);
+      __syncwarp();
+      iters = 0;
+    }
+  }
+  __syncwarp();
+  if (lane == 0) iacc_fold(acc[w]);
+  nn = warp_sum_ll((long long)nn); np = warp_sum_ll((long long)np); nm = warp_sum_ll((long long)nm);
+  if (lane == 0) {
+    if (nn) atomicAdd(&out->n_nan, nn);
+    if (np) atomicAdd(&out->n_pinf, np);
+    if (nm) atomicAdd(&out->n_ninf, nm);
+  }
+  __syncthreads();
+  // one global add per limb and block: |sum| < IACC_WARPS * 2^32 per block (limb 67 excepted, which stays small) and the
+  // grid is a few thousand blocks, so the global limbs cannot overflow; the host folds their carries
+  for (int j = threadIdx.x; j < IACC_LIMBS; j += blockDim.x) {
+    long long s = 0;
+    for (int v = 0; v < IACC_WARPS; ++v) s += acc[v][j];
+    iacc_add(out->limb, j, s);
+  }
+}

@@ -48,6 +48,7 @@ const char* kTaskNames[MPASB200_T_COUNT] = {
 std::string g_create_error;
 
 struct HaloList { int entity; int n; int* d_idx; };
+struct Weights { int entity; int n; double* d_w; };      // mpasb200_register_weights, caller's numbering
 
 }  // namespace
 
@@ -99,6 +100,7 @@ struct mpasb200 {
   std::vector<HaloList> lists;
   int* d_gid[3] = {nullptr, nullptr, nullptr}; int n_gid[3] = {0, 0, 0};   // mpasb200_set_global_ids
   SumAcc* d_acc = nullptr;
+  std::vector<Weights> weights; IntAcc* d_iacc = nullptr; double* d_wv = nullptr;   // mpasb200_integrate
   // distributed step (mpasb200_dist_*): NCCL communicator, halo lists, packed buffers, communication stream
   void* comm = nullptr; int rank = 0, world = 1;
   struct Halo { std::vector<int> peers_s, off_s, peers_r, off_r; int* d_s = nullptr; int* d_r = nullptr; int ns = 0, nr = 0; bool set = false; } halo[3];
@@ -961,6 +963,9 @@ int mpasb200_destroy(mpasb200_t* h) {
   if (h->h_stage) cudaFreeHost(h->h_stage);
   for (int e = 0; e < 3; ++e) if (h->d_gid[e]) cudaFree(h->d_gid[e]);
   if (h->d_acc) cudaFree(h->d_acc);
+  for (auto& w : h->weights) if (w.d_w) cudaFree(w.d_w);
+  if (h->d_iacc) cudaFree(h->d_iacc);
+  if (h->d_wv) cudaFree(h->d_wv);
   if (h->d_sflux) cudaFree(h->d_sflux);
   dist_release(h);
   for (auto& pp : h->pipe) {
@@ -1892,6 +1897,131 @@ int mpasb200_summarize_field(mpasb200_t* h, int field, int32_t n_first, int32_t 
   out->max_index = any ? (int64_t)(a.loc_max / (unsigned long long)nlevels) : -1; out->max_level = any ? (int32_t)(a.loc_max % (unsigned long long)nlevels) : -1;
   out->n_nan = (int64_t)a.n_nan; out->n_inf = (int64_t)a.n_inf; out->count = (int64_t)total; out->checksum = a.checksum;
   return 0;
+}
+
+// ---- exact global integrals (k_integrate) ------------------------------------------------------------------------------------------
+static_assert(IACC_LIMBS == MPASB200_INTEGRAL_LIMBS && IACC_BIAS == MPASB200_INTEGRAL_BIAS, "k_integrate and mpas_b200.h disagree");
+int mpasb200_register_weights(mpasb200_t* h, int entity, const double* w, int32_t n, int32_t* weight_id) {
+  REQUIRE_MESH();
+  if (entity < 0 || entity > MPASB200_VERTEX || !w || !weight_id) return fail(h, MPASB200_EINVAL, "register_weights: bad argument");
+  std::unique_lock<std::mutex> lk(h->mu);
+  cudaSetDevice(h->device);
+  if (n != entity_count(h, entity)) return fail(h, MPASB200_EINVAL, "register_weights: n is not the entity count");
+  Weights x{entity, n, nullptr};
+  CK(cudaMalloc((void**)&x.d_w, sizeof(double) * std::max(n, 1)));
+  h->weights.push_back(x);                    // before the copy, so that destroy frees it whatever happens next
+  if (n > 0) CK(cudaMemcpy(x.d_w, w, sizeof(double) * n, cudaMemcpyHostToDevice));
+  *weight_id = (int32_t)h->weights.size() - 1;
+  return 0;
+}
+int mpasb200_integrate(mpasb200_t* h, int field_a, int slot_a, int field_b, int slot_b, int weight_id, const double* wv,
+                       int32_t n_first, int32_t nlevels, MpasIntegral* out) {
+  REQUIRE_MESH();
+  if (!out || field_a < 0 || field_a >= MPASB200_F_COUNT || field_b < -1 || field_b >= MPASB200_F_COUNT)
+    return fail(h, MPASB200_EINVAL, "integrate: bad argument");
+  const FieldInfo& fa = kFields[field_a];
+  if (fa.entity == MPASB200_VERTICAL) return fail(h, MPASB200_EINVAL, "integrate: a vertical field");
+  if (slot_a < 0 || slot_a >= fa.slots) return fail(h, MPASB200_EINVAL, "integrate: slot_a out of range");
+  if (field_b >= 0) {
+    if (kFields[field_b].entity != fa.entity) return fail(h, MPASB200_EINVAL, "integrate: field_b lives on another entity type");
+    if (slot_b < 0 || slot_b >= kFields[field_b].slots) return fail(h, MPASB200_EINVAL, "integrate: slot_b out of range");
+  }
+  std::unique_lock<std::mutex> lk(h->mu);
+  cudaSetDevice(h->device);
+  if (h->capturing) return fail(h, MPASB200_ESTATE, "integrate during graph capture");
+  if (weight_id < -1 || weight_id >= (int)h->weights.size()) return fail(h, MPASB200_EINVAL, "integrate: unknown weight_id");
+  if (weight_id >= 0 && h->weights[weight_id].entity != fa.entity) return fail(h, MPASB200_EINVAL, "integrate: weights on another entity type");
+  const int n = entity_count(h, fa.entity);
+  if (n_first < 0 || n_first > n || nlevels < 1 || nlevels > h->L1) return fail(h, MPASB200_EINVAL, "integrate: range");
+  const size_t slotStride = (size_t)(n + 1) * h->LP;          // array-typed fields: slots one after the other (as pack)
+  const double* pa = h->V.f[field_a] + slot_a * slotStride;
+  const double* pb = field_b >= 0 ? h->V.f[field_b] + slot_b * slotStride : nullptr;
+  const double* pw = weight_id >= 0 ? h->weights[weight_id].d_w : nullptr;
+  if (!h->d_iacc) CK(cudaMalloc((void**)&h->d_iacc, sizeof(IntAcc)));
+  if (wv && !h->d_wv) CK(cudaMalloc((void**)&h->d_wv, sizeof(double) * h->L1));
+  if (wv) CK(cudaMemcpyAsync(h->d_wv, wv, sizeof(double) * nlevels, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemsetAsync(h->d_iacc, 0, sizeof(IntAcc), h->stream));
+  const size_t total = (size_t)n_first * nlevels;
+  if (total > 0) {
+    const int tpb = 32 * IACC_WARPS;
+    const int blocks = (int)std::min<size_t>((total + tpb - 1) / tpb, (size_t)h->num_sms * 8);
+    KTimer kt_(h, "k_integrate");
+    k_integrate<<<blocks, tpb, 0, h->stream>>>(pa, pb, h->d_newOf[fa.entity], pw, wv ? h->d_wv : nullptr, n_first, nlevels, h->LP, h->d_iacc);
+    h->launches++;
+    CK(cudaGetLastError());
+  }
+  IntAcc a;
+  CK(cudaMemcpyAsync(&a, h->d_iacc, sizeof(a), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));                        // also keeps wv borrowed for the call only
+  MpasIntegral r{};
+  for (int j = 0; j < IACC_LIMBS; ++j) r.limb[j] = a.limb[j];
+  r.count = (int64_t)total; r.n_nan = (int64_t)a.n_nan; r.n_pinf = (int64_t)a.n_pinf; r.n_ninf = (int64_t)a.n_ninf;
+  *out = MpasIntegral{};
+  return mpasb200_integral_merge(out, &r);                     // the canonical form
+}
+
+namespace {
+// exact canonical form of sum_j t[j] * 2^(32 j - BIAS): limbs 0..66 in [0, 2^32), the rest (signed) returned as the top
+__int128 integral_canon(const __int128* t, int64_t* limb) {
+  __int128 c = 0;
+  for (int j = 0; j < MPASB200_INTEGRAL_LIMBS - 1; ++j) {
+    const __int128 v = t[j] + c;
+    limb[j] = (int64_t)(v & 0xffffffff);
+    c = (v - limb[j]) / ((__int128)1 << 32);                    // exact: v - limb[j] is a multiple of 2^32
+  }
+  return t[MPASB200_INTEGRAL_LIMBS - 1] + c;
+}
+}  // namespace
+
+int mpasb200_integral_merge(MpasIntegral* acc, const MpasIntegral* x) {
+  if (!acc || !x) return MPASB200_EINVAL;
+  __int128 t[MPASB200_INTEGRAL_LIMBS];
+  for (int j = 0; j < MPASB200_INTEGRAL_LIMBS; ++j) t[j] = (__int128)acc->limb[j] + x->limb[j];
+  int64_t limb[MPASB200_INTEGRAL_LIMBS];
+  const __int128 top = integral_canon(t, limb);
+  if (top > INT64_MAX || top < INT64_MIN) return MPASB200_EINVAL;    // |sum| >= 2^1119 (no library result gets near): acc unchanged
+  limb[MPASB200_INTEGRAL_LIMBS - 1] = (int64_t)top;
+  std::memcpy(acc->limb, limb, sizeof(limb));
+  acc->count += x->count; acc->n_nan += x->n_nan; acc->n_pinf += x->n_pinf; acc->n_ninf += x->n_ninf;
+  return 0;
+}
+
+double mpasb200_integral_value(const MpasIntegral* x) {
+  constexpr int NL = MPASB200_INTEGRAL_LIMBS;
+  if (!x || x->n_nan || (x->n_pinf && x->n_ninf)) return NAN;
+  if (x->n_pinf) return INFINITY;
+  if (x->n_ninf) return -INFINITY;
+  __int128 t[NL];
+  int64_t limb[NL];
+  for (int j = 0; j < NL; ++j) t[j] = x->limb[j];
+  __int128 top = integral_canon(t, limb);
+  const bool neg = top < 0;
+  if (neg) {                                                     // the magnitude: negate limb by limb, then canonicalise again
+    for (int j = 0; j < NL - 1; ++j) t[j] = -(__int128)limb[j];
+    t[NL - 1] = -top;
+    top = integral_canon(t, limb);                              // now >= 0
+  }
+  // the magnitude as base-2^32 digits: limbs 0..66, then the 128-bit top in four digits
+  uint32_t d[NL + 3];
+  for (int j = 0; j < NL - 1; ++j) d[j] = (uint32_t)limb[j];
+  for (int j = 0; j < 4; ++j) d[NL - 1 + j] = (uint32_t)((unsigned __int128)top >> (32 * j));
+  int hi = NL + 2;
+  while (hi >= 0 && d[hi] == 0) --hi;
+  if (hi < 0) return 0.0;                                        // an exact zero is +0
+  auto bit = [&](int b) { return (d[b >> 5] >> (b & 31)) & 1u; };
+  const int msb = 32 * hi + 31 - __builtin_clz(d[hi]);            // bit index of the leading one
+  const int e_msb = msb - MPASB200_INTEGRAL_BIAS;
+  if (e_msb > 1023) return neg ? -INFINITY : INFINITY;
+  const int lsb = std::max(e_msb - 52, -1074);                  // weight of the last bit a double keeps (subnormals: 2^-1074)
+  const int q = lsb + MPASB200_INTEGRAL_BIAS;                    // >= 14
+  uint64_t m = 0;
+  for (int b = msb; b >= q; --b) m = (m << 1) | bit(b);
+  bool sticky = false;                                          // any one below the rounding bit q - 1
+  for (int j = 0; j < ((q - 1) >> 5) && !sticky; ++j) sticky = d[j] != 0;
+  sticky = sticky || (d[(q - 1) >> 5] & ((1u << ((q - 1) & 31)) - 1u)) != 0;
+  if (bit(q - 1) && (sticky || (m & 1))) ++m;                    // to nearest, ties to even
+  const double r = std::ldexp((double)m, lsb);                  // exact, or +inf when rounding reached 2^1024
+  return neg ? -r : r;
 }
 
 // ---- the distributed step ----------------------------------------------------------------------------------------------------

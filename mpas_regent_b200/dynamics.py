@@ -103,6 +103,11 @@ def _declare(lib, prefix: str, handle_t=C.c_void_p):
         lib.mpasb200_set_global_ids.argtypes, lib.mpasb200_set_global_ids.restype = [H, I, C.c_void_p, C.c_int32], I
         lib.mpasb200_summarize_field.argtypes = [H, I, C.c_int32, C.c_int32, C.POINTER(_abi.MpasFieldSummary)]
         lib.mpasb200_summarize_field.restype = I
+        lib.mpasb200_register_weights.argtypes = [H, I, C.c_void_p, C.c_int32, C.POINTER(C.c_int32)]
+        lib.mpasb200_integrate.argtypes = [H, I, I, I, I, I, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(_abi.MpasIntegral)]
+        lib.mpasb200_integral_merge.argtypes = [C.POINTER(_abi.MpasIntegral), C.POINTER(_abi.MpasIntegral)]
+        lib.mpasb200_integral_value.argtypes, lib.mpasb200_integral_value.restype = [C.POINTER(_abi.MpasIntegral)], D
+        lib.mpasb200_register_weights.restype = lib.mpasb200_integrate.restype = lib.mpasb200_integral_merge.restype = I
         lib.mpasb200_dist_unique_id.argtypes, lib.mpasb200_dist_unique_id.restype = [C.c_void_p], I
         lib.mpasb200_dist_init.argtypes, lib.mpasb200_dist_init.restype = [H, I, I, C.c_void_p], I
         lib.mpasb200_dist_set_halo.argtypes = [H, I, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -437,6 +442,30 @@ class Dynamics(TaskAPI):
         self._check(self._lib.mpasb200_summarize_field(self._h, FIELD_ID[name], n, nl, C.byref(out)), "summarize_field")
         return out.as_dict()
 
+    # ---- exact global integrals (mpasb200_integrate) ------------------------------------------------------------
+    def register_weights(self, entity: int, w: np.ndarray) -> int:
+        """upload a per-entity weight (caller's numbering, one value per local entity) once; returns its id"""
+        w = np.ascontiguousarray(w, dtype=np.float64)
+        wid = C.c_int32(-1)
+        self._check(self._lib.mpasb200_register_weights(self._h, entity, w.ctypes.data, w.shape[0], C.byref(wid)), "register_weights")
+        return int(wid.value)
+
+    def integrate(self, a: str, slot_a: int = 0, b: Optional[str] = None, slot_b: int = 0, weight_id: Optional[int] = None,
+                  wv: Optional[np.ndarray] = None, n_first: Optional[int] = None, nlevels: Optional[int] = None) -> dict:
+        """the exact sum of ((a * b) * wh[i]) * wv[k] over the first ``n_first`` entities (default all) and levels
+        [0, nlevels) (default all nVertLevels+1), non-finite products counted and left out (mpas_b200.h); see integral_result"""
+        n = self.entity_count(FIELD_ENTITY[a]) if n_first is None else int(n_first)
+        nl = self.dims.nVertLevels + 1 if nlevels is None else int(nlevels)
+        if wv is not None:
+            wv = np.ascontiguousarray(wv, dtype=np.float64)
+            if wv.shape != (nl,):
+                raise ValueError(f"wv: shape {wv.shape}, expected ({nl},)")
+        out = _abi.MpasIntegral()
+        self._check(self._lib.mpasb200_integrate(self._h, FIELD_ID[a], int(slot_a), -1 if b is None else FIELD_ID[b], int(slot_b),
+                                                 -1 if weight_id is None else int(weight_id), None if wv is None else wv.ctypes.data,
+                                                 n, nl, C.byref(out)), "integrate")
+        return integral_result(out)
+
     # ---- the distributed step inside the library (mpasb200_dist_*) --------------------------------------------
     @staticmethod
     def dist_unique_id() -> bytes:
@@ -544,6 +573,30 @@ class Dynamics(TaskAPI):
             self._check(self._lib.mpasb200_task_time(self._h, t, C.byref(ms), C.byref(calls), C.byref(nm)), "task_time")
             out[nm.value.decode()] = (ms.value, calls.value)
         return out
+
+
+def integral_result(acc: _abi.MpasIntegral) -> dict:
+    """an MpasIntegral as {value (rounded once), bits (of value, 16 hex digits), count, n_nan, n_pinf, n_ninf, limbs (int64[68])}"""
+    v = float(load_library().mpasb200_integral_value(C.byref(acc)))
+    return {"value": v, "bits": f"{int(np.float64(v).view(np.uint64)):016x}", "count": int(acc.count), "n_nan": int(acc.n_nan),
+            "n_pinf": int(acc.n_pinf), "n_ninf": int(acc.n_ninf), "limbs": np.array(acc.limb[:], dtype=np.int64)}
+
+
+def as_integral(r: dict) -> _abi.MpasIntegral:
+    """the MpasIntegral of an integral_result dict (limbs and counts; the value is derived)"""
+    acc = _abi.MpasIntegral()
+    acc.limb[:] = [int(x) for x in r["limbs"]]
+    acc.count, acc.n_nan, acc.n_pinf, acc.n_ninf = (int(r[k]) for k in ("count", "n_nan", "n_pinf", "n_ninf"))
+    return acc
+
+
+def merge_integrals(parts: Iterable[dict]) -> dict:
+    """exact merge of integral_result dicts (mpasb200_integral_merge: the order of ``parts`` does not matter)"""
+    lib, acc = load_library(), _abi.MpasIntegral()
+    for r in parts:
+        if lib.mpasb200_integral_merge(C.byref(acc), C.byref(as_integral(r))) != 0:
+            raise MpasB200Error("mpasb200_integral_merge: the sum leaves the accumulator's range")
+    return integral_result(acc)
 
 
 def dims_of(mesh, nVertLevels: int) -> MpasDims:

@@ -30,7 +30,7 @@ import numpy as np
 
 from . import _abi, partition
 from ._abi import CELL, EDGE, FIELD_ENTITY, FIELD_SLOTS, VERTEX
-from .dynamics import TaskAPI
+from .dynamics import TaskAPI, merge_integrals as _merge_integrals
 
 ENT = {"cell": CELL, "edge": EDGE, "vertex": VERTEX}
 
@@ -407,6 +407,27 @@ class DistributedDynamics:
 
 
 # ---- shards --------------------------------------------------------------------------------------------------
+def merge_integrals(parts: Sequence[dict], dist=None) -> dict:
+    """Exact global integral from per-partition ones (Dynamics.integrate over each partition's owned entities).  ``parts``
+    are the results this process holds; with ``dist`` (torch.distributed, initialised) every process's parts are gathered
+    first, limbs as int64 arrays, so no float enters the merge and every rank returns the same bits."""
+    parts = list(parts)
+    if dist is not None and dist.get_world_size() > 1:
+        every = [None] * dist.get_world_size()
+        dist.all_gather_object(every, parts)
+        parts = [p for ps in every for p in ps]
+    return _merge_integrals(parts)
+
+
+def column_integrals(dyn, area_id: int, n_owned: Optional[int] = None, dist=None, fields: Sequence[str] = ("rho_zz", "ke")) -> dict:
+    """{field: exact integral of field x areaCell x (1/rdzw)} over the first ``n_owned`` cells (default all) and levels
+    0..nVertLevels-1, merged over ranks (merge_integrals): the total mass for rho_zz.  ``area_id`` = the handle's
+    register_weights(CELL, areaCell of the rows it holds)."""
+    L = dyn.dims.nVertLevels
+    dz = 1.0 / dyn.download_field("rdzw")[:L]
+    return {f: merge_integrals([dyn.integrate(f, weight_id=area_id, wv=dz, n_first=n_owned, nlevels=L)], dist) for f in fields}
+
+
 def make_static_shards(st, world: int, colours: Optional[np.ndarray] = None):
     """partition the level-0 data of a HostState (CORRECTED policy; init_jw.make_static is enough, no 3-D field is read)
     into per-rank {lm, static}, launch classes included."""

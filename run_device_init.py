@@ -13,8 +13,9 @@ atm_srk3 on one GPU) with bench.dt_for(nCells).  bench.py itself keeps the host-
 
 Prints one JSON line: init seconds (host mesh / level-0 data, shard loading, device), peak host RSS per rank, ms per step,
 bench.run_check's combined checksum over owned entities (identical at every N when the N-rank state is bit-identical to
-the single-partition one), and the name and power limit of the card (read, never set).  --time-make-state also times, on
-rank 0 after everything else (so the peak RSS above is the device path's), the host generator bench.py uses for the same
+the single-partition one), the total mass (rho_zz x areaCell x 1/rdzw) and the same integral of ke, exact and merged
+over ranks (parallel.column_integrals: the same bits at every N), and the name and power limit of the card (read, never
+set).  --time-make-state also times, on rank 0 after everything else (so the peak RSS above is the device path's), the host generator bench.py uses for the same
 mesh (icosa mesh + init_jw.make_state), for comparison with the init seconds.
 """
 import argparse
@@ -117,6 +118,7 @@ def main():
     g = dynamics.Dynamics(_abi.make_dims(*n_loc, L), cfg)
     g.set_stream(stream.cuda_stream)
     g.upload_mesh(sh["static"])
+    area_id = g.register_weights(_abi.CELL, sh["jw"]["areaCell"])
     g.sync(); torch.cuda.synchronize()
     t2 = time.perf_counter()
     with torch.cuda.stream(stream):
@@ -152,6 +154,7 @@ def main():
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
         check = bench.run_check(g, lm, dist, world)
+        integrals = parallel.column_integrals(g, area_id, None if lm is None else lm.n_owned[0], dist if world > 1 else None)
     mine = {"ms": ms, "t_load": t_load, "t_dev": t_dev, "rss_gb": resource.getrusage(resource.RUSAGE_SELF).ru_maxrss / 2 ** 20,
             "card": card(local_rank)}
     ranks = [mine]
@@ -174,6 +177,8 @@ def main():
                            "device_max": round(max(r["t_dev"] for r in ranks), 3)},
                 "peak_host_rss_gb": [round(r["rss_gb"], 3) for r in ranks],
                 "combined_checksum": check["combined_checksum"], "finite": check["finite"],
+                "integrals": {"what": "exact sum over owned cells and levels 0..L-1 of field x areaCell x (1/rdzw)",
+                              **{"mass" if f == "rho_zz" else f: {"value": r["value"], "bits": r["bits"]} for f, r in integrals.items()}},
                 "gpus": [r["card"] for r in ranks], "host_generator": host_gen}
         print(json.dumps(line), flush=True)
     g.close()
