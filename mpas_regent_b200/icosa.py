@@ -1,8 +1,10 @@
-"""Synthetic icosahedral Voronoi meshes of 10*4**n + 2 cells (BASELINE.json configs 2-5).
+"""Synthetic icosahedral Voronoi meshes of 10*4**n + 2 cells (BASELINE.json configs 2-5), and Voronoi meshes of
+arbitrary generators on the sphere.
 
 Deterministic and seedless: recursive bisection of the icosahedron gives the Delaunay
 triangulation (cells = triangulation points, Voronoi vertices = triangle circumcentres,
-nEdges = 3n-6, nVertices = 2n-4, 12 pentagons).  The output carries the same 38 variables,
+nEdges = 3n-6, nVertices = 2n-4, 12 pentagons).  ``make_voronoi_mesh`` takes the triangulation
+from the convex hull instead, so its cells may have anywhere from 3 to MAX_EDGES sides.  The output carries the same 38 variables,
 dimensions and conventions as the bundled ``x1.2562.grid.nc`` that ``load_mesh`` reads
 (reference: mesh_loading/mesh_loading.rg:123-201): 1-based ids, unit sphere, counter-
 clockwise ``edgesOnCell``/``verticesOnCell``/``cellsOnCell`` with edge i joining vertex i and
@@ -69,8 +71,10 @@ def _arc(a, b):
 
 
 def _tri_area(a, b, c):
-    """area of the spherical triangle (unit sphere), always >= 0."""
-    num = np.abs(np.einsum("ij,ij->i", a, np.cross(b, c)))
+    """signed area of the spherical triangle (unit sphere): positive when a, b, c run counter-clockwise seen from
+    outside.  A kite of a cell whose Voronoi vertex lies outside its triangle (an obtuse Delaunay triangle) is the sum
+    of one positive and one negative part; with unsigned parts the cell areas would no longer tile the sphere."""
+    num = np.einsum("ij,ij->i", a, np.cross(b, c))
     den = 1.0 + np.einsum("ij,ij->i", a, b) + np.einsum("ij,ij->i", b, c) + np.einsum("ij,ij->i", c, a)
     return 2.0 * np.arctan2(num, den)
 
@@ -124,8 +128,31 @@ def make_icosahedral_mesh(n_cells: int) -> Mesh:
     p, f = _icosahedron()
     for _ in range(lvl):
         p, f = _subdivide(p, f)
+    assert p.shape[0] == n_cells
+    m = mesh_from_triangulation(p, f, f"x1.{n_cells}")
+    deg = m.v["nEdgesOnCell"]
+    assert deg.min() == 5 and deg.max() <= 6 and int((deg == 5).sum()) == 12
+    return m
+
+
+def make_voronoi_mesh(points: np.ndarray, name: str) -> Mesh:
+    """The spherical Voronoi mesh of arbitrary generators (unit vectors, [n, 3]).  The convex hull of points on a sphere
+    is their spherical Delaunay triangulation; its faces are turned counter-clockwise seen from outside, as
+    ``_icosahedron`` does.  Cells may have 3 to MAX_EDGES sides."""
+    from scipy.spatial import ConvexHull
+    p = np.ascontiguousarray(points, dtype=np.float64)
+    f = ConvexHull(p).simplices.astype(np.int64)
+    a, b, c = p[f[:, 0]], p[f[:, 1]], p[f[:, 2]]
+    flip = np.einsum("ij,ij->i", np.cross(b - a, c - a), a + b + c) < 0
+    f[flip] = f[flip][:, [0, 2, 1]]
+    return mesh_from_triangulation(p, f, name)
+
+
+def mesh_from_triangulation(p: np.ndarray, f: np.ndarray, name: str) -> Mesh:
+    """The Voronoi mesh dual to a triangulation of the unit sphere: points ``p`` [nC, 3] become cells, the counter-
+    clockwise triangles ``f`` [nV, 3] (0-based) become vertices placed at their circumcentres."""
     nC, nV = p.shape[0], f.shape[0]
-    assert nC == n_cells and nV == 2 * nC - 4
+    assert nV == 2 * nC - 4
     nE = 3 * nC - 6
 
     # ---- directed half-edges: triangle t lies to the left of a->b; around a, b is followed by c
@@ -159,12 +186,12 @@ def make_icosahedral_mesh(n_cells: int) -> Mesh:
     first = np.searchsorted(a_s, np.arange(nC))           # first half-edge leaving each cell
     deg = np.searchsorted(a_s, np.arange(nC), side="right") - first
     nEdgesOnCell = deg.astype(np.int32)
-    assert deg.min() == 5 and deg.max() <= 6 and int((deg == 5).sum()) == 12
+    assert deg.min() >= 3 and deg.max() <= MAX_EDGES
     cellsOnCell = np.zeros((nC, MAX_EDGES), dtype=np.int64)
     triAfter = np.zeros((nC, MAX_EDGES), dtype=np.int64)   # triangle between neighbour i and i+1
     cur = b_s[first]
     me = np.arange(nC)
-    for i in range(6):
+    for i in range(int(deg.max())):
         act = i < deg
         pos = lookup(me, cur)
         cellsOnCell[act, i] = cur[act]
@@ -172,7 +199,7 @@ def make_icosahedral_mesh(n_cells: int) -> Mesh:
         cur = c_s[pos]
     edgesOnCell = np.zeros((nC, MAX_EDGES), dtype=np.int64)
     verticesOnCell = np.zeros((nC, MAX_EDGES), dtype=np.int64)
-    for i in range(6):
+    for i in range(int(deg.max())):
         act = i < deg
         edgesOnCell[act, i] = edge_of(me, cellsOnCell[:, i])[act]
         # vertex i sits before edge i (between edge i-1 and edge i)
@@ -240,6 +267,6 @@ def make_icosahedral_mesh(n_cells: int) -> Mesh:
         cellsOnCell=pad_last(cellsOnCell, deg), verticesOnCell=i32(voc), verticesOnEdge=i32(verticesOnEdge + 1),
         edgesOnVertex=i32(edgesOnVertex + 1), cellsOnVertex=i32(cellsOnVertex + 1), kiteAreasOnVertex=f64(kite),
     )
-    m = Mesh(v=v, partition=None, name=f"x1.{nC}")
+    m = Mesh(v=v, partition=None, name=name)
     m.validate()
     return m

@@ -51,6 +51,14 @@ def test_icosahedral_mesh_invariants(n):
     v = m.v
     assert m.nCells == n and m.nEdges == 3 * n - 6 and m.nVertices == 2 * n - 4
     assert int((v["nEdgesOnCell"] == 5).sum()) == 12
+    check_voronoi_invariants(m, trisk_edges=300)
+
+
+def check_voronoi_invariants(m, trisk_edges=None):
+    """what every closed spherical Voronoi mesh of the generator satisfies; TRiSK antisymmetry on the first
+    ``trisk_edges`` edges (all when None)."""
+    v = m.v
+    n = m.nCells
     for k in ("areaCell", "areaTriangle", "kiteAreasOnVertex"):
         assert abs(v[k].sum() - 4 * np.pi) < 1e-9
     # every edge appears once in each of its two cells; ids are 1-based
@@ -58,24 +66,53 @@ def test_icosahedral_mesh_invariants(n):
     slot = np.arange(10)[None, :] < ne[:, None]
     assert np.array_equal(np.bincount(eoc[slot] - 1, minlength=m.nEdges), np.full(m.nEdges, 2))
     assert v["cellsOnEdge"].min() == 1 and v["cellsOnEdge"].max() == n
-    # convention of the bundled file: edge i of a cell joins vertex i and vertex i+1
-    c = np.arange(n)
-    for i in range(5):
+    # convention of the bundled file: edge i of a cell joins vertex i and vertex i+1, for every slot up to the degree
+    for i in range(int(ne.max())):
+        c = np.flatnonzero(i < ne)
         e = eoc[c, i] - 1
         a = np.sort(v["verticesOnEdge"][e], axis=1)
-        nxt = np.where(i + 1 < ne, i + 1, 0)
+        nxt = np.where(i + 1 < ne[c], i + 1, 0)
         b = np.sort(np.stack([v["verticesOnCell"][c, i], v["verticesOnCell"][c, nxt]], 1), axis=1)
-        assert np.array_equal(a, b)
+        assert np.array_equal(a, b), i
     # TRiSK: weights are antisymmetric in energy norm  w_{e,e'} dc_e / dv_e' = - w_{e',e} dc_e' / dv_e
-    nE = m.nEdges
+    nE = m.nEdges if trisk_edges is None else min(m.nEdges, trisk_edges)
     W = {}
     eoe, woe, neoe = v["edgesOnEdge"] - 1, v["weightsOnEdge"], v["nEdgesOnEdge"]
-    for e in range(min(nE, 300)):
+    for e in range(nE):
         for j in range(neoe[e]):
             W[(e, eoe[e, j])] = woe[e, j] * v["dcEdge"][e] / v["dvEdge"][eoe[e, j]]
+    pairs = 0
     for (e, e2), w in W.items():
         if (e2, e) in W:
             assert abs(w + W[(e2, e)]) < 1e-12
+            pairs += 1
+    assert pairs > 0
+    if trisk_edges is None:
+        assert pairs == len(W)
+
+
+# SHA-256 over (name, dtype, shape, bytes) of every array, in name order, from the generator before it was split into
+# make_icosahedral_mesh + mesh_from_triangulation: the icosahedral meshes every other test runs on keep their bits.
+ICOSA_DIGESTS = {
+    642: "4efb030d31e3a27d1e402b51b6a910687107aa3491e2ef7a3b8ab880907dc0ed",
+    10242: "de069213bdd3173199773d13bb1888eda43267c7fb1e1fc651dcef561a91cff4",
+}
+
+
+def mesh_digest(m):
+    import hashlib
+    h = hashlib.sha256()
+    for k in sorted(m.v):
+        a = np.ascontiguousarray(m.v[k])
+        h.update(k.encode()); h.update(str(a.dtype).encode()); h.update(str(a.shape).encode()); h.update(a.tobytes())
+    return h.hexdigest()
+
+
+@pytest.mark.parametrize("n", sorted(ICOSA_DIGESTS))
+def test_icosahedral_mesh_bits_are_pinned(n):
+    m = icosa.make_icosahedral_mesh(n)
+    assert m.name == f"x1.{n}"
+    assert mesh_digest(m) == ICOSA_DIGESTS[n]
 
 
 def test_icosahedral_generator_is_deterministic():

@@ -158,7 +158,8 @@ def _numpy_acoustic_corrected(st, f, vert, cfg, dts, small_step):
     o["rtheta_pp_old"][:, K] = 0.0 if small_step == 0 else f["rtheta_pp"][:, K]
     if small_step == 0:
         rw_p[:] = 0; ww[:] = 0; rho_pp[:, K] = 0; rt_pp[:, K] = 0
-    assert np.all(s["specZoneMaskCell"] == 0.0)
+    spec = s["specZoneMaskCell"] != 0.0
+    before = [a[spec][:, K].copy() for a in (rho_pp, rt_pp, rw_p, ww)]
     rs, ts = np.zeros((nC, Lv)), np.zeros((nC, Lv))
     rup, tm = pad(o["ru_p"])[:, K], pad(f["theta_m"])[:, K]
     for i in range(s["edgesOnCell"].shape[1]):
@@ -190,16 +191,25 @@ def _numpy_acoustic_corrected(st, f, vert, cfg, dts, small_step):
     ww[:, k] += 0.5 * (1.0 + epssm) * rw_p[:, k]
     rho_pp[:, K] = rs - cofrz * (rw_p[:, 1:] - rw_p[:, :-1])
     rt_pp[:, K] = ts - rdzw * (coftz[:, 1:] * rw_p[:, 1:] - coftz[:, :-1] * rw_p[:, :-1])
+    # specified-zone columns only integrate their tendencies, every level from 0 (:1698-1703)
+    rho_pp[spec, K] = before[0] + dts * f["tend_rho"][spec][:, K]
+    rt_pp[spec, K] = before[1] + dts * f["theta_m"][spec][:, K]
+    rw_p[spec, K] = before[2] + dts * w[spec][:, K]
+    ww[spec, K] = before[3] + 0.5 * (1.0 + epssm) * rw_p[spec][:, K]
     return o
 
 
 @pytest.mark.parametrize("small_step", [0, 1])
 def test_corrected_physics_acoustic_step_matches_array_restatement(grid642, small_step):
-    st, lit, _ = build_pair(grid642, L, _abi.INDEX_CORRECTED, gpu=False)
+    check_corrected_acoustic_restatement(grid642, small_step)
+
+
+def check_corrected_acoustic_restatement(mesh, small_step, masks=None):
+    st, lit, _ = build_pair(mesh, L, _abi.INDEX_CORRECTED, gpu=False, masks=masks)
     lit.atm_compute_solve_diagnostics(False, -1)
     lit.atm_srk3(600.0)                                    # a finite, fully populated state
     pre = lit.download_all(); lit.close()
-    st, ora, _ = build_pair(grid642, L, _abi.INDEX_CORRECTED, gpu=False, physics_mode=_abi.PHYSICS_CORRECTED)
+    st, ora, _ = build_pair(mesh, L, _abi.INDEX_CORRECTED, gpu=False, masks=masks, physics_mode=_abi.PHYSICS_CORRECTED)
     for n, a in pre.items():
         ora.upload_field(n, a)
     ora.atm_advance_acoustic_step(300.0, small_step)

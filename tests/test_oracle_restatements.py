@@ -4,7 +4,7 @@ both must agree to rounding (1e-13 relative).  Memory-model rules as in the orac
 import numpy as np
 import pytest
 
-from mpas_regent_b200 import _abi
+from mpas_regent_b200 import _abi, dynamics
 from tests.util import build_pair
 
 L = 7
@@ -123,10 +123,11 @@ def test_advance_acoustic_step_literal(warmed, small_step):                 # dy
     rup, tm = _pad(f["ru_p"]), _pad(f["theta_m"])
     dv = np.append(s["dvEdge"], 0.0)
     zz, w = f["zz"], f["w"]
-    assert np.all(s["specZoneMaskCell"] == 0.0)
+    spec = s["specZoneMaskCell"] != 0.0
     for k in range(L):                                      # levels ascend (M4): level k sees the NEW level k-1
         if small_step == 0:
             rho_pp[:, k] = 0; rt_pp[:, k] = 0
+        before = [a[spec, k].copy() for a in (rho_pp, rt_pp, rw_p, ww)]
         rs, ts = np.zeros(nC), np.zeros(nC)
         for i in range(s["edgesOnCell"].shape[1]):
             on = i < s["nEdgesOnCell"]
@@ -152,6 +153,11 @@ def test_advance_acoustic_step_literal(warmed, small_step):                 # dy
             ww[:, k] += 0.5 * (1.0 + epssm) * rw_p[:, k]
         rho_pp[:, k] = rs - cofrz[k] * (rw_p[:, k + 1] - rw_p[:, k])
         rt_pp[:, k] = ts - rdzw[k] * (f["coftz"][:, k + 1] * rw_p[:, k + 1] - f["coftz"][:, k] * rw_p[:, k])
+        # specified-zone columns only integrate their tendencies (:1698-1703); level 0 included
+        rho_pp[spec, k] = before[0] + dts * f["tend_rho"][spec, k]
+        rt_pp[spec, k] = before[1] + dts * f["theta_m"][spec, k]
+        rw_p[spec, k] = before[2] + dts * w[spec, k]
+        ww[spec, k] = before[3] + 0.5 * (1.0 + epssm) * rw_p[spec, k]
     ora.atm_advance_acoustic_step(dts, small_step)
     _check(ora, o)
     assert np.abs(o["rw_p"]).max() > 0
@@ -159,10 +165,13 @@ def test_advance_acoustic_step_literal(warmed, small_step):                 # dy
 
 @pytest.mark.parametrize("fix", [False, True], ids=["literal", "corrected_physics"])
 @pytest.mark.parametrize("rk_step", [0, 2])
-def test_recover_large_step_variables(warmed, grid642, rk_step, fix):       # dynamics_tasks.rg:1786-1871, as written
+def test_recover_large_step_variables(warmed, rk_step, fix):                # dynamics_tasks.rg:1786-1871, as written
     st, ora, f = warmed
     if fix:        # MPASB200_PHYSICS_CORRECTED restores four expressions (include/mpas_b200.h)
-        st, ora, _ = build_pair(grid642, L, _abi.INDEX_CORRECTED, gpu=False, physics_mode=_abi.PHYSICS_CORRECTED)
+        from oracle.oracle import Oracle
+        ora = Oracle(dynamics.dims_of(st.mesh, L), _abi.default_config(index_policy=_abi.INDEX_CORRECTED, rkarg_policy=_abi.RKARG_STAGE_INDEX,
+                                                                      physics_mode=_abi.PHYSICS_CORRECTED))
+        ora.upload_mesh(st.static); ora.upload_state(st.f, st.vert)
     _reset(ora, f)
     s, cfg = st.static, ora.cfg
     nC, nE = s["nEdgesOnCell"].shape[0], s["cellsOnEdge"].shape[0]

@@ -225,7 +225,12 @@ def test_error_paths(grid642):
 def test_acoustic_modes(grid2562, exact):
     """every evaluation of the acoustic column sweep agrees with the oracle (1e-12); the strictly ordered ones
     (acoustic_exact=1, and the default acoustic_tma=3) are additionally bit-identical on the fields the sweep produces."""
-    st, ora, g = build_pair(grid2562, L_SMALL, _abi.INDEX_CORRECTED, m5=True, acoustic_exact=int(exact == 1), acoustic_tma=(exact - 1 if exact >= 2 else 0))
+    acoustic_mode_parity(grid2562, exact)
+
+
+def acoustic_mode_parity(mesh, exact, masks=None):
+    st, ora, g = build_pair(mesh, L_SMALL, _abi.INDEX_CORRECTED, m5=True, masks=masks, acoustic_exact=int(exact == 1),
+                            acoustic_tma=(exact - 1 if exact >= 2 else 0))
     _warm(ora, g)
     for b in (ora, g):
         for ss, dts in ((0, 360.0), (1, 360.0), (2, 360.0)):
@@ -318,14 +323,18 @@ def test_staged_gathers_bit_identical(grid2562, mask):
 def test_emulated_ranks_on_one_gpu_equal_single_partition(grid642, physics, split):
     """4 ranks emulated as 4 handles on one GPU (pack/unpack + the exchange schedule of parallel.exchanges_for):
     owned entities are bit-identical to the single-partition GPU run."""
+    from mpas_regent_b200 import init_jw
+    emulated_ranks_equal_single_partition(grid642, init_jw.make_state(grid642, 6, _abi.INDEX_CORRECTED), physics, split)
+
+
+def emulated_ranks_equal_single_partition(mesh, st, physics, split):
     import torch
-    from mpas_regent_b200 import dynamics, init_jw, parallel
+    from mpas_regent_b200 import dynamics, parallel
     from tests.test_parallel import _task_schedule, _assert_owned_equal
-    Lh = 6
-    st = init_jw.make_state(grid642, Lh, _abi.INDEX_CORRECTED)
+    Lh = st.nVertLevels
     cfg = _abi.default_config(rkarg_policy=_abi.RKARG_STAGE_INDEX, physics_mode=physics)
     exchanges = parallel.exchanges_for(cfg)
-    single = dynamics.Dynamics(dynamics.dims_of(grid642, Lh), cfg)
+    single = dynamics.Dynamics(dynamics.dims_of(mesh, Lh), cfg)
     single.upload_mesh(st.static); single.upload_state(st.f, st.vert)
     single.atm_compute_solve_diagnostics(False, -1)
     shards = parallel.make_shards(st, 4)
@@ -570,11 +579,15 @@ def test_range_restricted_launches_equal_whole(grid642, physics):
     """mpasb200_set_range: the acoustic step on cell ranges and the divergence damping on edge ranges, in any order of
     disjoint ranges that covers everything, give the bytes of the unrestricted launches; launch classes only permute the
     library's internal numbering."""
-    from mpas_regent_b200 import dynamics, init_jw
-    Lh = 9
-    st = init_jw.make_state(grid642, Lh, _abi.INDEX_CORRECTED)
+    from mpas_regent_b200 import init_jw
+    range_restricted_launches_equal_whole(grid642, init_jw.make_state(grid642, 9, _abi.INDEX_CORRECTED), physics)
+
+
+def range_restricted_launches_equal_whole(mesh, st, physics):
+    from mpas_regent_b200 import dynamics
+    Lh = st.nVertLevels
     cfg = _abi.default_config(rkarg_policy=_abi.RKARG_STAGE_INDEX, physics_mode=physics)
-    nC, nE = grid642.nCells, grid642.nEdges
+    nC, nE = mesh.nCells, mesh.nEdges
     rng = np.random.default_rng(11)
     outs = []
     for mode in ("whole", "ranges", "classes"):
@@ -582,7 +595,7 @@ def test_range_restricted_launches_equal_whole(grid642, physics):
         if mode == "classes":
             static["cellClass"] = rng.integers(0, 3, nC).astype(np.uint8)
             static["edgeClass"] = rng.integers(0, 2, nE).astype(np.uint8)
-        g = dynamics.Dynamics(dynamics.dims_of(grid642, Lh), cfg)
+        g = dynamics.Dynamics(dynamics.dims_of(mesh, Lh), cfg)
         g.upload_mesh(static); g.upload_state(st.f, st.vert)
         g.atm_compute_solve_diagnostics(False, -1)
         g.atm_srk3(500.0)                               # populate everything
@@ -621,12 +634,16 @@ from mpas_regent_b200._abi import CELL as parallel_CELL, EDGE as parallel_EDGE  
 def test_advance_scalars_parity(grid2562, policy):
     """the task alone on a state where everything it reads is non-trivial, then the driver with config_scalar_advection on
     (setup saves scalars_old, every RK stage advances; rk_timestep.rg:465), plain and as a CUDA graph: bit-identical."""
-    st, ora, g = build_pair(grid2562, L_SMALL, policy, m5=True, config_scalar_advection=1)
+    advance_scalars_parity(grid2562, policy)
+
+
+def advance_scalars_parity(mesh, policy, masks=None):
+    st, ora, g = build_pair(mesh, L_SMALL, policy, m5=True, masks=masks, config_scalar_advection=1)
     _warm(ora, g)
     rng = np.random.default_rng(9)
-    nC = grid2562.nCells
+    nC = mesh.nCells
     q = 1e-3 * (1.0 + rng.random((nC, L_SMALL + 1, 8))); q_old = 1e-3 * (1.0 + rng.random((nC, L_SMALL + 1, 8)))
-    ru = ora.download_field("ru") + 0.3 * rng.standard_normal((grid2562.nEdges, L_SMALL + 1))
+    ru = ora.download_field("ru") + 0.3 * rng.standard_normal((mesh.nEdges, L_SMALL + 1))
     ww = 0.05 * rng.standard_normal((nC, L_SMALL + 1))
     for b in (ora, g):
         for n, a in (("scalars", q), ("scalars_old", q_old), ("ruAvg", ru), ("wwAvg", ww)):
@@ -742,10 +759,13 @@ def test_mesh_only_init_producers_on_the_device(grid2562, grid642, policy, which
     """SURVEY.md 8f rank 3: atm_compute_signs (dynamics_tasks.rg:46-130), atm_adv_coef_compression (:133-269) and
     atm_couple_coef_3rd_order (:303-325) as device kernels, through the C ABI with the RAW stored ids: integer lists, signs and
     coefficients are bit-identical to the oracle's literal loops (and therefore to what the host chain fed every other test)."""
+    mesh_only_init_producers_equal_oracle(grid2562 if which == "x1.2562" else grid642, policy)
+
+
+def mesh_only_init_producers_equal_oracle(mesh, policy):
     from mpas_regent_b200 import dynamics, init_jw
     from oracle.oracle import Oracle
     from tests.test_core_init import _raw_mesh
-    mesh = grid2562 if which == "x1.2562" else grid642
     st = init_jw.make_state(mesh, L_SMALL, policy)
     raw = _raw_mesh(mesh, st.mesh, st.extras["deriv_two"])
     cfg = _abi.default_config(index_policy=policy)

@@ -6,10 +6,12 @@ from mpas_regent_b200 import _abi, dynamics, init_jw
 TOL = 1e-12   # BASELINE.json north_star: "within 1e-12 relative (fp64) per field"
 
 
-def build_pair(mesh, L, policy, m5=True, gpu=True, rkarg=_abi.RKARG_STAGE_INDEX, sfc=1, **cfg_over):
-    """(state, oracle, gpu-or-None) with identical mesh + fields uploaded."""
+def build_pair(mesh, L, policy, m5=True, gpu=True, rkarg=_abi.RKARG_STAGE_INDEX, sfc=1, masks=None, **cfg_over):
+    """(state, oracle, gpu-or-None) with identical mesh + fields uploaded; ``masks`` replaces level-0 arrays of the state
+    (the regional masks bdyMaskCell, specZoneMaskCell, specZoneMaskEdge, isShared)."""
     from oracle.oracle import Oracle
     st = init_jw.make_state(mesh, L, policy, m5=m5)
+    st.static.update(masks or {})
     dims = dynamics.dims_of(mesh, L)
     cfg = _abi.default_config(index_policy=policy, rkarg_policy=rkarg, sfc_renumber=sfc, **cfg_over)
     ora = Oracle(dims, cfg)
