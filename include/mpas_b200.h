@@ -383,6 +383,31 @@ int  mpasb200_integrate(mpasb200_t *h, int field_a, int slot_a, int field_b, int
 int  mpasb200_integral_merge(MpasIntegral *acc, const MpasIntegral *x);
 double mpasb200_integral_value(const MpasIntegral *x);
 
+/* ---- surface pressure and pressure-level diagnostics ------------------------------------------------------------------- *
+ * Column-local, so the owned rows of N ranks equal the single handle's rows bit for bit.  For cell c (the device mirror as
+ * it is at the call), L = nVertLevels, mass levels k = 0..L-1, w-levels 0..L, ln = the device's log():
+ *   p(k)    = pressure_base(k) + pressure_p(k)
+ *   T(k)    = theta_m(k) * exner(k)                              (dry: qtot = 0, theta = theta_m)
+ *   z(k)    = 0.5 * (zgrid(k) + zgrid(k+1))
+ *   wm(k)   = 0.5 * (w(k) + w(k+1))
+ *   uzon(k), umer(k) = the zonal / meridional wind of mpas_reconstruct_2d (on_a_sphere = 1) at level k, in its expressions
+ *             and order; uReconstruct* are NOT written (atm_compute_dyn_tend reads uReconstructZonal/Meridional)
+ *   zeta(k) = num / den,  num = sum_i a_i * vorticity(v_i, k),  den = sum_i a_i,  i = 0..nEdgesOnCell-1 in slot order,
+ *             both sums from 0.0, left to right; v_i = verticesOnCell[c][i], a_i = kiteAreasOnVertex[v_i][kiteForCell[c][i]]
+ *             (the kite-weighted mean of the vertex vorticity)
+ *   ps      = p(0) + (zgrid(0) - z(0)) * ((p(1) - p(0)) / (z(1) - z(0)))      (linear in height from the two lowest levels)
+ * For each requested pressure P (Pa): k* = the SMALLEST k in 0..L-2 with p(k) >= P and P >= p(k+1) (comparisons with NaN are
+ * false).  No such k (P below the lowest or above the highest mass level, non-finite columns): all six values are NaN.
+ * Otherwise a = 1 if p(k*) == p(k*+1), else (ln P - ln p(k*+1)) / (ln p(k*) - ln p(k*+1)), and
+ * f = f(k*+1) + a * (f(k*) - f(k*+1)) for f in T, z, uzon, umer, wm, zeta.  Everything else is IEEE arithmetic (the library
+ * is built with --fmad=false, so only a goes through a libm call).
+ * out = [n_first][1 + 6*nplev] doubles in the caller's cell numbering: out[i][0] = ps, then per level j: T, z, uzon, umer,
+ * wm, zeta.  plev may be in any order and may repeat.  The call is synchronous and refused during graph capture
+ * (MPASB200_ESTATE); MPASB200_EINVAL for a null out or plev, nplev outside [1, MPASB200_ISOBARIC_MAX_LEVELS], a plev entry
+ * that is not finite or not > 0, n_first outside [0, nCells].                                                             */
+#define MPASB200_ISOBARIC_MAX_LEVELS 32
+int  mpasb200_isobaric_diagnostics(mpasb200_t *h, const double *plev, int32_t nplev, int32_t n_first, double *out);
+
 /* ---- halo exchange building blocks (one process per GPU; the wire is the host's job) ------ *
  * Lists are LOCAL entity indices in the caller's (un-renumbered) numbering.  pack gathers
  * `n` columns x `nfields` fields x (nVertLevels+1) levels into the contiguous device

@@ -120,6 +120,12 @@ class MpasIntegral(C.Structure):
                 ("n_ninf", C.c_int64)]
 
 
+#: mpasb200_isobaric_diagnostics: at most this many pressure levels per call; each output row is surface pressure, then per
+#: level these six values in this order
+ISOBARIC_MAX_LEVELS = 32
+ISOBARIC_FIELDS = ("temperature", "height", "uzonal", "umeridional", "w", "vorticity")
+
+
 INIT_MESH_MEMBERS = (
     ("nEdgesOnCell", np.int32, CELL, 1), ("edgesOnCell", np.int32, CELL, "maxEdges"), ("verticesOnCell", np.int32, CELL, "maxEdges"),
     ("cellsOnCell", np.int32, CELL, "maxEdges"), ("cellsOnEdge", np.int32, EDGE, 2), ("verticesOnEdge", np.int32, EDGE, 2),

@@ -2031,23 +2031,34 @@ __global__ void k_icd_cell2(const View V, double rgas, double rcv) {
   st2m(FLD(pressure_p), ix, zz * rgas * (ex * rtp + rtb * (ex - exb)), m0, m1);
   st2m(FLD(pressure_base), ix, zz * rgas * exb * rtb, m0, m1);
 }
-// mpas_reconstruct_2d  :1894-1948
+// mpas_reconstruct_2d  :1894-1948, the arithmetic of one cell, shared by k_reconstruct and k_isobaric.  T = D2 (a level pair)
+// or double; ue(e) = u of edge e at the level(s).
+template <class T, class Ue> DI void recon_xyz(const View& V, int x, Ue ue, T& ux, T& uy, T& uz) {
+  const int ME = V.maxEdges, n = V.nEdgesOnCell[x];
+  ux = T{}; uy = T{}; uz = T{};
+  for (int i = 0; i < n; ++i) {
+    const T u = ue(V.edgesOnCell[x * V.MEP + i]);
+    const double* cf = V.coeffsRecon + ((size_t)x * ME + i) * 3;
+    ux += cf[0] * u; uy += cf[1] * u; uz += cf[2] * u;
+  }
+}
+template <class T> DI void recon_sphere(const View& V, int x, T ux, T uy, T uz, T& zonal, T& meridional) {   // on_a_sphere
+  const double clat = V.cosLatCell[x], slat = V.sinLatCell[x], clon = V.cosLonCell[x], slon = V.sinLonCell[x];
+  zonal = -ux * slon + uy * clon;
+  meridional = -(ux * clon + uy * slon) * slat + uz * clat;
+}
 __global__ void k_reconstruct(const View V, int on_a_sphere) {
   PAIR_THREAD(V.nCells)
   if (!m0) return;
-  const int ME = V.maxEdges, n = V.nEdgesOnCell[x];
   const double* u = FLD(u);
-  D2 ux = bc(0.0), uy = bc(0.0), uz = bc(0.0);
-  for (int i = 0; i < n; ++i) {
-    const D2 ue = G2(u, V.edgesOnCell[x * V.MEP + i]);
-    const double* cf = V.coeffsRecon + ((size_t)x * ME + i) * 3;
-    ux += cf[0] * ue; uy += cf[1] * ue; uz += cf[2] * ue;
-  }
+  D2 ux, uy, uz;
+  recon_xyz(V, x, [&](int e) { return G2(u, e); }, ux, uy, uz);
   st2m(FLD(uReconstructX), ix, ux, m0, m1); st2m(FLD(uReconstructY), ix, uy, m0, m1); st2m(FLD(uReconstructZ), ix, uz, m0, m1);
   if (on_a_sphere) {
-    const double clat = V.cosLatCell[x], slat = V.sinLatCell[x], clon = V.cosLonCell[x], slon = V.sinLonCell[x];
-    st2m(FLD(uReconstructZonal), ix, -ux * slon + uy * clon, m0, m1);
-    st2m(FLD(uReconstructMeridional), ix, -(ux * clon + uy * slon) * slat + uz * clat, m0, m1);
+    D2 zonal, meridional;
+    recon_sphere(V, x, ux, uy, uz, zonal, meridional);
+    st2m(FLD(uReconstructZonal), ix, zonal, m0, m1);
+    st2m(FLD(uReconstructMeridional), ix, meridional, m0, m1);
   } else {
     st2m(FLD(uReconstructZonal), ix, ux, m0, m1); st2m(FLD(uReconstructMeridional), ix, uy, m0, m1);
   }
@@ -2150,6 +2161,74 @@ __global__ void k_summarize_loc(const double* __restrict__ field, const int* __r
     if (key == kmin) atomicMin(&acc->loc_min, id);
     if (key == kmax) atomicMin(&acc->loc_max, id);
   }
+}
+
+// ============================================================================================
+// Surface pressure and pressure-level diagnostics (mpasb200_isobaric_diagnostics; mpas_b200.h states the definition).
+// One warp per cell of the caller's first n cells.  The lanes read the pressure column 32 levels at a time (levels are
+// contiguous, so each chunk is one coalesced strip), and one ballot per target and chunk finds the first bracket of every
+// target.  Lane j then handles target j and gathers only its level pair (k*, k*+1): theta_m, exner, w and zgrid up to k*+2,
+// u on the cell's edges and vorticity on its vertices.  Nothing but `out` is written.
+struct IsoLevels { double p[MPASB200_ISOBARIC_MAX_LEVELS]; int n; };
+constexpr int ISO_WARPS = 8;            // blockDim.x = 32 * ISO_WARPS
+__global__ void __launch_bounds__(32 * ISO_WARPS)
+k_isobaric(const View V, const int* __restrict__ map, const IsoLevels P, int n, double* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const int i = blockIdx.x * ISO_WARPS + (threadIdx.x >> 5);
+  if (i >= n) return;                                    // warp-uniform
+  const int x = map[i], L = V.L, LP = V.LP, np = P.n;
+  const size_t col = (size_t)x * LP;
+  const double* pb = FLD(pressure_base) + col; const double* pp = FLD(pressure_p) + col;
+  const double* zg = FLD(zgrid) + col;
+  int ks = -1;                                           // lane j < np: k* of target j
+  for (int c = 0; c < L - 1; c += 32) {
+    const int k = c + lane;
+    const double pk = k < L ? pb[k] + pp[k] : 0.0;
+    double pk1 = __shfl_down_sync(0xffffffffu, pk, 1);
+    if (lane == 31 && k + 1 < L) pk1 = pb[k + 1] + pp[k + 1];
+    const bool live = k <= L - 2;
+    for (int j = 0; j < np; ++j) {
+      const double t = P.p[j];
+      const unsigned b = __ballot_sync(0xffffffffu, live && pk >= t && t >= pk1);
+      if (lane == j && ks < 0 && b) ks = c + __ffs(b) - 1;
+    }
+  }
+  double* row = out + (size_t)i * (1 + 6 * np);
+  if (lane == 0) {
+    const double p0 = pb[0] + pp[0], p1 = pb[1] + pp[1];
+    const double z0 = 0.5 * (zg[0] + zg[1]), z1 = 0.5 * (zg[1] + zg[2]);
+    row[0] = p0 + (zg[0] - z0) * ((p1 - p0) / (z1 - z0));
+  }
+  if (lane >= np) return;
+  double* o = row + 1 + 6 * lane;
+  if (ks < 0) {
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    for (int q = 0; q < 6; ++q) o[q] = nan;
+    return;
+  }
+  const int k = ks;
+  const double* th = FLD(theta_m) + col; const double* ex = FLD(exner) + col; const double* w = FLD(w) + col;
+  const double* u = FLD(u); const double* vo = FLD(vorticity);
+  const double t = P.p[lane], pa = pb[k] + pp[k], pz = pb[k + 1] + pp[k + 1];
+  const double a = pa == pz ? 1.0 : (log(t) - log(pz)) / (log(pa) - log(pz));
+  // level pairs (k*, k*+1): .x = k*, .y = k*+1
+  const D2 T = mk(th[k] * ex[k], th[k + 1] * ex[k + 1]);
+  const D2 z = mk(0.5 * (zg[k] + zg[k + 1]), 0.5 * (zg[k + 1] + zg[k + 2]));
+  const D2 wm = mk(0.5 * (w[k] + w[k + 1]), 0.5 * (w[k + 1] + w[k + 2]));
+  D2 ux, uy, uz, uzon, umer;
+  recon_xyz(V, x, [&](int e) { return mk(u[(size_t)e * LP + k], u[(size_t)e * LP + k + 1]); }, ux, uy, uz);
+  recon_sphere(V, x, ux, uy, uz, uzon, umer);
+  const int ME = V.maxEdges, ne = V.nEdgesOnCell[x];
+  D2 num = bc(0.0);
+  double den = 0.0;
+  for (int s = 0; s < ne; ++s) {
+    const int v = V.verticesOnCell[x * ME + s];
+    const double ar = V.kiteAreasOnVertex[v * V.vertexDegree + V.kiteForCell[x * ME + s]];
+    num += ar * mk(vo[(size_t)v * LP + k], vo[(size_t)v * LP + k + 1]); den += ar;
+  }
+  const D2 zeta = num / den;
+  const D2 f[6] = {T, z, uzon, umer, wm, zeta};
+  for (int q = 0; q < 6; ++q) o[q] = f[q].y + a * (f[q].x - f[q].y);
 }
 
 // ============================================================================================

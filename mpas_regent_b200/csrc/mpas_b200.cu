@@ -101,6 +101,7 @@ struct mpasb200 {
   int* d_gid[3] = {nullptr, nullptr, nullptr}; int n_gid[3] = {0, 0, 0};   // mpasb200_set_global_ids
   SumAcc* d_acc = nullptr;
   std::vector<Weights> weights; IntAcc* d_iacc = nullptr; double* d_wv = nullptr;   // mpasb200_integrate
+  double* d_iso = nullptr; size_t iso_elems = 0;      // mpasb200_isobaric_diagnostics output, grown on demand
   // distributed step (mpasb200_dist_*): NCCL communicator, halo lists, packed buffers, communication stream
   void* comm = nullptr; int rank = 0, world = 1;
   struct Halo { std::vector<int> peers_s, off_s, peers_r, off_r; int* d_s = nullptr; int* d_r = nullptr; int ns = 0, nr = 0; bool set = false; } halo[3];
@@ -966,6 +967,7 @@ int mpasb200_destroy(mpasb200_t* h) {
   for (auto& w : h->weights) if (w.d_w) cudaFree(w.d_w);
   if (h->d_iacc) cudaFree(h->d_iacc);
   if (h->d_wv) cudaFree(h->d_wv);
+  if (h->d_iso) cudaFree(h->d_iso);
   if (h->d_sflux) cudaFree(h->d_sflux);
   dist_release(h);
   for (auto& pp : h->pipe) {
@@ -1896,6 +1898,39 @@ int mpasb200_summarize_field(mpasb200_t* h, int field, int32_t n_first, int32_t 
   out->min_index = any ? (int64_t)(a.loc_min / (unsigned long long)nlevels) : -1; out->min_level = any ? (int32_t)(a.loc_min % (unsigned long long)nlevels) : -1;
   out->max_index = any ? (int64_t)(a.loc_max / (unsigned long long)nlevels) : -1; out->max_level = any ? (int32_t)(a.loc_max % (unsigned long long)nlevels) : -1;
   out->n_nan = (int64_t)a.n_nan; out->n_inf = (int64_t)a.n_inf; out->count = (int64_t)total; out->checksum = a.checksum;
+  return 0;
+}
+
+// ---- surface pressure and pressure-level diagnostics (k_isobaric) ---------------------------------------------------------------
+int mpasb200_isobaric_diagnostics(mpasb200_t* h, const double* plev, int32_t nplev, int32_t n_first, double* out) {
+  REQUIRE_MESH();
+  if (!out || !plev) return fail(h, MPASB200_EINVAL, "isobaric_diagnostics: null out or plev");
+  if (nplev < 1 || nplev > MPASB200_ISOBARIC_MAX_LEVELS) return fail(h, MPASB200_EINVAL, "isobaric_diagnostics: nplev outside [1, 32]");
+  IsoLevels P{};
+  P.n = nplev;
+  for (int j = 0; j < nplev; ++j) {
+    if (!std::isfinite(plev[j]) || !(plev[j] > 0.0)) return fail(h, MPASB200_EINVAL, "isobaric_diagnostics: a plev entry is not finite and > 0");
+    P.p[j] = plev[j];
+  }
+  if (n_first < 0 || n_first > h->nCells) return fail(h, MPASB200_EINVAL, "isobaric_diagnostics: n_first outside [0, nCells]");
+  std::unique_lock<std::mutex> lk(h->mu);
+  cudaSetDevice(h->device);
+  if (h->capturing) return fail(h, MPASB200_ESTATE, "isobaric_diagnostics during graph capture");
+  const size_t elems = (size_t)n_first * (1 + 6 * nplev);
+  if (elems == 0) return 0;
+  if (h->iso_elems < elems) {
+    if (h->d_iso) { CK(cudaFree(h->d_iso)); h->d_iso = nullptr; h->iso_elems = 0; }
+    CK(cudaMalloc((void**)&h->d_iso, sizeof(double) * elems));
+    h->iso_elems = elems;
+  }
+  {
+    KTimer kt_(h, "k_isobaric");
+    k_isobaric<<<(n_first + ISO_WARPS - 1) / ISO_WARPS, 32 * ISO_WARPS, 0, h->stream>>>(h->V, h->d_newOf[MPASB200_CELL], P, n_first, h->d_iso);
+    h->launches++;
+  }
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(out, h->d_iso, sizeof(double) * elems, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
   return 0;
 }
 

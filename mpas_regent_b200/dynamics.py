@@ -108,6 +108,8 @@ def _declare(lib, prefix: str, handle_t=C.c_void_p):
         lib.mpasb200_integral_merge.argtypes = [C.POINTER(_abi.MpasIntegral), C.POINTER(_abi.MpasIntegral)]
         lib.mpasb200_integral_value.argtypes, lib.mpasb200_integral_value.restype = [C.POINTER(_abi.MpasIntegral)], D
         lib.mpasb200_register_weights.restype = lib.mpasb200_integrate.restype = lib.mpasb200_integral_merge.restype = I
+        lib.mpasb200_isobaric_diagnostics.argtypes = [H, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]
+        lib.mpasb200_isobaric_diagnostics.restype = I
         lib.mpasb200_dist_unique_id.argtypes, lib.mpasb200_dist_unique_id.restype = [C.c_void_p], I
         lib.mpasb200_dist_init.argtypes, lib.mpasb200_dist_init.restype = [H, I, I, C.c_void_p], I
         lib.mpasb200_dist_set_halo.argtypes = [H, I, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -465,6 +467,24 @@ class Dynamics(TaskAPI):
                                                  -1 if weight_id is None else int(weight_id), None if wv is None else wv.ctypes.data,
                                                  n, nl, C.byref(out)), "integrate")
         return integral_result(out)
+
+    # ---- surface pressure and pressure-level diagnostics (mpasb200_isobaric_diagnostics) ------------------------------
+    def isobaric_diagnostics(self, plev_pa, n_first: Optional[int] = None) -> Dict[str, np.ndarray]:
+        """surface pressure and T, height, zonal / meridional wind, w and vorticity on the pressure surfaces ``plev_pa`` (Pa,
+        any order, repeats allowed) for the first ``n_first`` cells (default all), computed on the device from the mirror as
+        it is (mpas_b200.h states the definition; NaN where a level is not bracketed by the column).  Returns
+        {"surface_pressure": [n], "temperature" | "height" | "uzonal" | "umeridional" | "w" | "vorticity": [n, len(plev_pa)]}."""
+        plev = np.ascontiguousarray(np.atleast_1d(np.asarray(plev_pa, dtype=np.float64)))
+        if plev.ndim != 1:
+            raise ValueError(f"plev_pa: shape {plev.shape}, expected one dimension")
+        n = self.dims.nCells if n_first is None else int(n_first)
+        P = plev.shape[0]
+        out = np.empty((max(n, 0), 1 + 6 * P), dtype=np.float64)
+        self._check(self._lib.mpasb200_isobaric_diagnostics(self._h, plev.ctypes.data, P, n, out.ctypes.data), "isobaric_diagnostics")
+        r = {"surface_pressure": out[:, 0].copy()}
+        for q, name in enumerate(_abi.ISOBARIC_FIELDS):
+            r[name] = np.ascontiguousarray(out[:, 1 + q::6])
+        return r
 
     # ---- the distributed step inside the library (mpasb200_dist_*) --------------------------------------------
     @staticmethod

@@ -428,6 +428,35 @@ def column_integrals(dyn, area_id: int, n_owned: Optional[int] = None, dist=None
     return {f: merge_integrals([dyn.integrate(f, weight_id=area_id, wv=dz, n_first=n_owned, nlevels=L)], dist) for f in fields}
 
 
+def isobaric_diagnostics(dyn, lm, plev_pa, dist=None) -> Optional[Dict[str, np.ndarray]]:
+    """Dynamics.isobaric_diagnostics of the owned cells of every rank, assembled in global cell order on rank 0 (other ranks
+    get None).  ``dyn`` / ``lm`` are this rank's handle and LocalMesh (``lm`` None: one rank holding the whole mesh), or
+    equal-length lists of them for ranks emulated in one process; with ``dist`` (torch.distributed, initialised) the rows
+    travel to rank 0 over it.  The values are column-local, so the assembled arrays have the same bits at every rank count."""
+    dyns, lms = (list(dyn), list(lm)) if isinstance(dyn, (list, tuple)) else ([dyn], [lm])
+    parts = []
+    for d, m in zip(dyns, lms):
+        n = d.dims.nCells if m is None else m.n_owned[0]
+        cells = np.arange(n) if m is None else np.asarray(m.cells[:n])
+        parts.append((cells, d.isobaric_diagnostics(plev_pa, n_first=n)))
+    if dist is not None and dist.get_world_size() > 1:
+        every = [None] * dist.get_world_size() if dist.get_rank() == 0 else None
+        dist.gather_object(parts, every, dst=0)
+        if dist.get_rank() != 0:
+            return None
+        parts = [p for ps in every for p in ps]
+    n = sum(len(c) for c, _ in parts)
+    out = {k: np.empty((n,) + v.shape[1:], dtype=np.float64) for k, v in parts[0][1].items()}
+    seen = np.zeros(n, dtype=bool)
+    for cells, r in parts:
+        seen[cells] = True
+        for k, v in r.items():
+            out[k][cells] = v
+    if not seen.all():
+        raise ValueError("isobaric_diagnostics: the ranks' owned cells do not cover the mesh")
+    return out
+
+
 def make_static_shards(st, world: int, colours: Optional[np.ndarray] = None):
     """partition the level-0 data of a HostState (CORRECTED policy; init_jw.make_static is enough, no 3-D field is read)
     into per-rank {lm, static}, launch classes included."""

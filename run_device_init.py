@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """run_device_init.py -- every rank builds its shard of the initial state on its own GPU, then runs the RK3 step.
 
-    python run_device_init.py [--mesh CELLS] [--levels L] [--steps K] [--warmup W]                 (one GPU)
-    torchrun --nproc-per-node N run_device_init.py [--mesh CELLS] [--levels L] [--steps K] [--warmup W]
+    python run_device_init.py [--mesh CELLS] [--levels L] [--steps K] [--warmup W] [--plev HPA,...]  (one GPU)
+    torchrun --nproc-per-node N run_device_init.py [--mesh CELLS] [--levels L] [--steps K] [--warmup W] [--plev HPA,...]
 
 Rank 0 builds the mesh and the level-0 data only (init_jw.make_static: no 3-D array exists on the host) and partitions it
 (parallel.make_static_shards); the shards are staged as .npy files in a temporary directory (under /dev/shm when there is
@@ -15,11 +15,14 @@ Prints one JSON line: init seconds (host mesh / level-0 data, shard loading, dev
 bench.run_check's combined checksum over owned entities (identical at every N when the N-rank state is bit-identical to
 the single-partition one), the total mass (rho_zz x areaCell x 1/rdzw) and the same integral of ke, exact and merged
 over ranks (parallel.column_integrals: the same bits at every N), and the name and power limit of the card (read, never
-set).  --time-make-state also times, on rank 0 after everything else (so the peak RSS above is the device path's), the host generator bench.py uses for the same
+set).  --plev HPA[,HPA...] adds one parallel.isobaric_diagnostics call after the timed steps: its ms (on rank 0, assembly in
+global cell order included), per level the min and max of the temperature, the min of the surface pressure and a SHA-256
+of the assembled arrays (the same string at every N).  --time-make-state also times, on rank 0 after everything else (so the peak RSS above is the device path's), the host generator bench.py uses for the same
 mesh (icosa mesh + init_jw.make_state), for comparison with the init seconds.
 """
 import argparse
 import datetime
+import hashlib
 import json
 import os
 import resource
@@ -57,10 +60,18 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--time-make-state", action="store_true", help="also time the host generator (make_state) on rank 0")
+    ap.add_argument("--plev", type=str, default=None, help="pressure levels in hPa, comma-separated: one isobaric_diagnostics call")
     args = ap.parse_args()
     if args.steps < 1:
         ap.error("--steps must be at least 1")
+    plev_hpa = None
+    if args.plev is not None:
+        try:
+            plev_hpa = [float(x) for x in args.plev.split(",")]
+        except ValueError:
+            ap.error("--plev: comma-separated numbers (hPa)")
 
+    import numpy as np
     import torch
     from mpas_regent_b200 import _abi, dynamics, icosa, init_jw, parallel
 
@@ -155,6 +166,20 @@ def main():
         ms = e0.elapsed_time(e1)
         check = bench.run_check(g, lm, dist, world)
         integrals = parallel.column_integrals(g, area_id, None if lm is None else lm.n_owned[0], dist if world > 1 else None)
+        isobaric = None
+        if plev_hpa is not None:
+            t5 = time.perf_counter()
+            iso = parallel.isobaric_diagnostics(g, lm, [100.0 * p for p in plev_hpa], dist if world > 1 else None)
+            t_iso = time.perf_counter() - t5
+            if iso is not None:
+                digest = hashlib.sha256(iso["surface_pressure"].tobytes())
+                for name in _abi.ISOBARIC_FIELDS:
+                    digest.update(iso[name].tobytes())
+                T = iso["temperature"]
+                isobaric = {"plev_hpa": plev_hpa, "ms": round(1e3 * t_iso, 3), "ps_min": float(np.nanmin(iso["surface_pressure"])),
+                            "T_min": [float(np.nanmin(T[:, j])) if np.isfinite(T[:, j]).any() else None for j in range(T.shape[1])],
+                            "T_max": [float(np.nanmax(T[:, j])) if np.isfinite(T[:, j]).any() else None for j in range(T.shape[1])],
+                            "sha256": digest.hexdigest()}
     mine = {"ms": ms, "t_load": t_load, "t_dev": t_dev, "rss_gb": resource.getrusage(resource.RUSAGE_SELF).ru_maxrss / 2 ** 20,
             "card": card(local_rank)}
     ranks = [mine]
@@ -180,6 +205,8 @@ def main():
                 "integrals": {"what": "exact sum over owned cells and levels 0..L-1 of field x areaCell x (1/rdzw)",
                               **{"mass" if f == "rho_zz" else f: {"value": r["value"], "bits": r["bits"]} for f, r in integrals.items()}},
                 "gpus": [r["card"] for r in ranks], "host_generator": host_gen}
+        if isobaric is not None:
+            line["isobaric"] = isobaric
         print(json.dumps(line), flush=True)
     g.close()
     if world > 1:
