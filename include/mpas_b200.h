@@ -408,6 +408,15 @@ double mpasb200_integral_value(const MpasIntegral *x);
 #define MPASB200_ISOBARIC_MAX_LEVELS 32
 int  mpasb200_isobaric_diagnostics(mpasb200_t *h, const double *plev, int32_t nplev, int32_t n_first, double *out);
 
+/* ---- the restart set ------------------------------------------------------------------------------------------------- *
+ * The fields a restart must hold under `cfg` (mpas_b200_restart.def): every mirror field whose value at a step boundary can
+ * change a later step, and the ones the step never rewrites.  Every other field is rewritten by each step before it is read,
+ * so a fresh handle (mpasb200_create, upload_mesh) into which these fields are uploaded continues bit for bit like the handle
+ * they were downloaded from, at a step boundary (after mpasb200_dist_flush), at any rank count.  Writes the ids of the first
+ * min(count, cap) of them to `ids` (may be null when cap <= 0) in the order of the .def file and returns the count; needs no
+ * handle and no GPU.  MPASB200_EINVAL for a null cfg.                                                                      */
+int  mpasb200_restart_fields(const MpasConfig *cfg, int32_t *ids, int32_t cap);
+
 /* ---- halo exchange building blocks (one process per GPU; the wire is the host's job) ------ *
  * Lists are LOCAL entity indices in the caller's (un-renumbered) numbering.  pack gathers
  * `n` columns x `nfields` fields x (nVertLevels+1) levels into the contiguous device

@@ -53,6 +53,31 @@ FIELD_SLOTS: Dict[str, int] = {n: s for (n, _, s) in FIELDS}
 N_FIELDS = len(FIELDS)
 
 
+RESTART_WHEN = ("ALWAYS", "CORRECTED", "SCALARS")
+
+
+def _parse_restart() -> List[Tuple[str, str]]:
+    out = []
+    with open(os.path.join(INCLUDE_DIR, "mpas_b200_restart.def")) as fh:
+        for line in fh:
+            m = re.match(r"\s*MPASB200_RESTART\(\s*(\w+)\s*,\s*(\w+)\s*\)", line)
+            if m:
+                if m.group(1) not in FIELD_ID or m.group(2) not in RESTART_WHEN:
+                    raise ValueError(f"mpas_b200_restart.def: bad line {line.strip()}")
+                out.append((m.group(1), m.group(2)))
+    return out
+
+
+#: include/mpas_b200_restart.def: (field, when) in file order
+RESTART: List[Tuple[str, str]] = _parse_restart()
+
+
+def restart_fields(cfg: "MpasConfig") -> List[str]:
+    """the restart set under ``cfg``, in the order of mpasb200_restart_fields"""
+    on = {"ALWAYS": True, "CORRECTED": cfg.physics_mode == PHYSICS_CORRECTED, "SCALARS": cfg.config_scalar_advection != 0}
+    return [n for n, when in RESTART if on[when]]
+
+
 class MpasDims(C.Structure):
     _fields_ = [(n, C.c_int32) for n in
                 ("nCells", "nEdges", "nVertices", "nVertLevels", "maxEdges", "maxEdges2", "vertexDegree", "nAdvCells")]

@@ -2142,6 +2142,17 @@ int mpasb200_field_by_name(const char* name) {
   for (int i = 0; i < MPASB200_F_COUNT; ++i) if (!std::strcmp(name, kFields[i].name)) return i;
   return -1;
 }
+int mpasb200_restart_fields(const MpasConfig* cfg, int32_t* ids, int32_t cap) {
+  if (!cfg) return MPASB200_EINVAL;
+  const bool ALWAYS = true, CORRECTED = cfg->physics_mode == MPASB200_PHYSICS_CORRECTED, SCALARS = cfg->config_scalar_advection != 0;
+  (void)CORRECTED;
+  int32_t n = 0;
+#define MPASB200_RESTART(name, when) \
+  if (when) { if (ids && n < cap) ids[n] = MPASB200_F_##name; ++n; }
+#include "../../include/mpas_b200_restart.def"
+#undef MPASB200_RESTART
+  return n;
+}
 #ifdef MPASB200_LAB
 // Experimental launch variants of the divergence-damping kernel (not part of the public header): used by
 // profiles/ scripts to measure latency-hiding structures.  variant 0 = production kernel.

@@ -110,6 +110,8 @@ def _declare(lib, prefix: str, handle_t=C.c_void_p):
         lib.mpasb200_register_weights.restype = lib.mpasb200_integrate.restype = lib.mpasb200_integral_merge.restype = I
         lib.mpasb200_isobaric_diagnostics.argtypes = [H, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]
         lib.mpasb200_isobaric_diagnostics.restype = I
+        lib.mpasb200_restart_fields.argtypes = [C.POINTER(MpasConfig), C.c_void_p, C.c_int32]
+        lib.mpasb200_restart_fields.restype = I
         lib.mpasb200_dist_unique_id.argtypes, lib.mpasb200_dist_unique_id.restype = [C.c_void_p], I
         lib.mpasb200_dist_init.argtypes, lib.mpasb200_dist_init.restype = [H, I, I, C.c_void_p], I
         lib.mpasb200_dist_set_halo.argtypes = [H, I, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]

@@ -17,7 +17,10 @@ the single-partition one), the total mass (rho_zz x areaCell x 1/rdzw) and the s
 over ranks (parallel.column_integrals: the same bits at every N), and the name and power limit of the card (read, never
 set).  --plev HPA[,HPA...] adds one parallel.isobaric_diagnostics call after the timed steps: its ms (on rank 0, assembly in
 global cell order included), per level the min and max of the temperature, the min of the surface pressure and a SHA-256
-of the assembled arrays (the same string at every N).  --time-make-state also times, on rank 0 after everything else (so the peak RSS above is the device path's), the host generator bench.py uses for the same
+of the assembled arrays (the same string at every N).  --restart DIR skips the device init and resumes from a restart (mpas_regent_b200/restart.py, written at any rank count); the
+steps then continue its step count.  --save-restart DIR writes one after the timed steps.  A run resumed from a restart of
+K steps and run for M more prints the same checksum, integrals and isobaric SHA-256 as an uninterrupted run of K + M steps.
+--time-make-state also times, on rank 0 after everything else (so the peak RSS above is the device path's), the host generator bench.py uses for the same
 mesh (icosa mesh + init_jw.make_state), for comparison with the init seconds.
 """
 import argparse
@@ -61,6 +64,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--time-make-state", action="store_true", help="also time the host generator (make_state) on rank 0")
     ap.add_argument("--plev", type=str, default=None, help="pressure levels in hPa, comma-separated: one isobaric_diagnostics call")
+    ap.add_argument("--save-restart", type=str, default=None, metavar="DIR", help="write a restart (restart.save) after the timed steps")
+    ap.add_argument("--restart", type=str, default=None, metavar="DIR", help="skip the device init and resume from a restart (restart.load)")
     args = ap.parse_args()
     if args.steps < 1:
         ap.error("--steps must be at least 1")
@@ -73,7 +78,7 @@ def main():
 
     import numpy as np
     import torch
-    from mpas_regent_b200 import _abi, dynamics, icosa, init_jw, parallel
+    from mpas_regent_b200 import _abi, dynamics, icosa, init_jw, parallel, restart
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -95,10 +100,13 @@ def main():
     # ---- host: mesh and level-0 data on rank 0 only, one shard per rank ----
     t0 = time.perf_counter()
     lm = None
+    keep_mesh = args.restart is not None or args.save_restart is not None      # restart.save / load check it (rank 0)
+    mesh_global = None
     if world == 1:
         mesh = icosa.make_icosahedral_mesh(nC)
         st, draws = init_jw.make_static(mesh, L, _abi.INDEX_CORRECTED)
         sh = dict(static=st.static, vert=st.vert, jw=init_jw.jw_inputs(mesh, st, draws))
+        mesh_global = mesh if keep_mesh else None
         del mesh, st, draws
         t_host = time.perf_counter() - t0
         t_load = 0.0
@@ -111,6 +119,7 @@ def main():
             for r, s in enumerate(parallel.make_static_shards(st, world)):
                 s.update(vert=st.vert, jw=init_jw.jw_inputs(mesh, st, draws, s["lm"]))
                 parallel.save_shard(os.path.join(stage, f"rank{r}"), s)
+            mesh_global = mesh if keep_mesh else None
             del mesh, st, draws, s
             box = [stage]
         dist.broadcast_object_list(box, src=0)
@@ -132,15 +141,22 @@ def main():
     area_id = g.register_weights(_abi.CELL, sh["jw"]["areaCell"])
     g.sync(); torch.cuda.synchronize()
     t2 = time.perf_counter()
+    step0 = 0
     with torch.cuda.stream(stream):
-        init_jw.init_on_device(g, sh["static"], sh["jw"], sh["vert"])
+        if args.restart is not None:
+            step0 = restart.load(args.restart, g, lm, mesh_global, dist)
+        else:
+            init_jw.init_on_device(g, sh["static"], sh["jw"], sh["vert"])
         if world > 1:
-            parallel.NcclExchanger(g, lm, stream).exchange(parallel.INIT_EXCHANGE)
+            if args.restart is None:
+                parallel.NcclExchanger(g, lm, stream).exchange(parallel.INIT_EXCHANGE)
             run = parallel.NativeDistributedDynamics(g, lm, rank, world)
-            run.init_diagnostics()
+            if args.restart is None:
+                run.init_diagnostics()
             step = lambda: run.step(dt)
         else:
-            g.atm_compute_solve_diagnostics(False, -1)
+            if args.restart is None:
+                g.atm_compute_solve_diagnostics(False, -1)
             step = lambda: g.atm_srk3(dt)
         g.sync(); torch.cuda.synchronize()
     t_dev = time.perf_counter() - t2
@@ -164,6 +180,11 @@ def main():
         e1.record(stream)
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
+        t_save = None
+        if args.save_restart is not None:
+            t6 = time.perf_counter()
+            restart.save(args.save_restart, g, lm, step0 + args.warmup + args.steps, mesh_global, dist)
+            t_save = time.perf_counter() - t6
         check = bench.run_check(g, lm, dist, world)
         integrals = parallel.column_integrals(g, area_id, None if lm is None else lm.n_owned[0], dist if world > 1 else None)
         isobaric = None
@@ -197,6 +218,8 @@ def main():
     if rank == 0:
         line = {"what": "device-built initial state (init_jw.init_on_device per rank) + RK3 steps", "mesh": nC, "levels": L,
                 "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "dt": dt,
+                "step_count": step0 + args.warmup + args.steps, "restart_from": args.restart,
+                "restart_save_s": None if t_save is None else round(t_save, 3),
                 "ms_per_step": max(r["ms"] for r in ranks) / args.steps,
                 "init_s": {"host_mesh_static": round(t_host, 3), "shard_load_max": round(max(r["t_load"] for r in ranks), 3),
                            "device_max": round(max(r["t_dev"] for r in ranks), 3)},
